@@ -23,9 +23,13 @@ Timed region (SURVEY.md 8d "steady state: >= 100 back-to-back forward calls"; VE
     own request first, pbg_score_triplets);
   * inputs rotate over a pool of pre-staged batches larger than L2; every pool entry is executed once before timing;
   * each lane's rotation over its pool entries is ONE CUDA graph; the timed region replays the lanes' graphs
-    back to back: `steps` x `repeats` passes inside one CUDA-event pair, `repeats` chosen so that the region lasts
-    >= 50 ms (K = 20 alone is 0.4 ms: ramp and tail, not throughput); the region is measured `trials` times and
-    the MEDIAN is the headline (`best` beside it);
+    back to back: exactly `steps` passes (step j runs pool entry j mod pool size) inside one CUDA-event pair, issued
+    behind a short spin kernel so that the region times the GPU and not the host's launches; the region is measured
+    `trials` times and the MEDIAN is the headline (`best` beside it).  A short region includes the ramp and the tail
+    of the lanes: pick `steps` large enough for the figure wanted (a 4096-triplet step took ~24 us on a B200 at its
+    1000 W power limit, DESIGN.md section 4);
+  * `--dump-outputs DIR` writes what the last timed step returned (gen_out, gen_scores, logits, probs; float32 .npy):
+    the inputs depend only on the arguments, so two builds can be compared output for output;
   * NVML clocks are sampled every 10 ms during the trials by a thread that does nothing else.
 
 Printed JSON (one line, rank 0):
@@ -51,6 +55,7 @@ import time
 from pathlib import Path
 
 os.environ.setdefault("CUDA_DEVICE_MAX_CONNECTIONS", "32")   # lanes x (compute + ingest) streams: no false serialisation
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree it runs from
 
 ROOT = Path(__file__).resolve().parent
 for p in (str(ROOT / "pro-b-gan_b200"), str(ROOT)):
@@ -61,6 +66,10 @@ import torch  # noqa: E402
 
 NUM_ENTITIES, NUM_RELATIONS = 65536, 64
 L2_BYTES = 126 * 2 ** 20
+DUMP_MAX_BYTES = 64 * 2 ** 20
+DUMP_SAMPLE_SEED = 2024
+SPIN_CYCLES = 2_000_000   # ~1 ms of SM clock: longer than the host takes to issue the first launches of a region
+SUSTAINED_MIN_MS = 25.0   # timed regions at least this long are compared with the sustained (power-capped) peak
 METRIC = "generator+discriminator samples/sec (score_triplets pass, bf16 tensor-core mode)"
 CONFIGS = {
     "base": {"E": 128, "Z": 64, "H": 1024, "batch": 4096,
@@ -98,6 +107,27 @@ def make_models(cfg: dict, gen_cls, disc_cls):
     if cfg["H"] == 1024:
         return synth.make_models(gen_cls, disc_cls, cfg["E"], cfg["Z"], cfg["H"])
     return synth.make_models(gen_cls, disc_cls, cfg["E"], cfg["Z"], cfg["H"], cfg["H"])
+
+
+def dump_outputs(out_dir: str, arrays: dict) -> None:
+    """Writes {name: tensor, one row per triplet} as out_dir/<name>.npy in float32.  Above DUMP_MAX_BYTES the same
+    fixed, seeded sample of rows is kept in every array, and the row numbers go to rows.npy (float64)."""
+    import numpy as np
+    arrays = {k: v.detach().float().cpu() for k, v in arrays.items()}
+    rows = next(iter(arrays.values())).shape[0]
+    row_bytes = sum(v[:1].numel() * 4 for v in arrays.values())
+    if rows * row_bytes > DUMP_MAX_BYTES:
+        keep = (DUMP_MAX_BYTES - 128 * (len(arrays) + 1)) // (row_bytes + 8)   # 128 B per .npy header, 8 B per row number
+        idx = torch.randperm(rows, generator=torch.Generator().manual_seed(DUMP_SAMPLE_SEED))[:keep].sort().values
+        arrays = {k: v[idx] for k, v in arrays.items()}
+        arrays["rows"] = idx.double()
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(d / f"{k}.npy", v.numpy())
+
+
+OUTPUT_NAMES = ("gen_out", "gen_scores", "logits", "probs")
 
 
 # ------------------------------------------------------------------------------------------ CPU oracle leg
@@ -153,8 +183,10 @@ def run_reference(args, cfg: dict, rank: int, world: int) -> None:
         fn()
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        fn()
+        res = fn()
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(zip(OUTPUT_NAMES, res)))
     value = sample * args.steps / dt
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": "samples/s", "n_gpus": args.gpus,
@@ -526,28 +558,24 @@ def run_b200(args, cfg: dict, rank: int, local_rank: int, world: int) -> None:
             tail_cache[rem] = capture([[x for x in lane_entries[l] if x < rem] for l in range(S)])
         return tail_cache[rem]
 
-    # ---- warm-up (graphs executed at least once, >= W steps) and calibration of `repeats`
+    # ---- warm-up (graphs executed at least once, >= W steps), then `trials` timed regions of exactly K steps
     def timed(n_steps: int) -> float:
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         torch.cuda.synchronize(); barrier()
+        torch.cuda._sleep(SPIN_CYCLES)   # the region starts once the host has issued its first launches behind it
         ev0.record(main)
         issue(n_steps, full_graphs, tail_graphs_for)
         ev1.record(main)
         torch.cuda.synchronize(); barrier()
         return ev0.elapsed_time(ev1)
 
+    n_timed = K
     warm_steps = max(W, 2 * P)
-    if use_graphs and (K * 1) % P:
-        tail_graphs_for((K * 1) % P)   # capture outside any timed region
-    ms_warm = max_over_ranks(timed(warm_steps))
-    est_step = ms_warm / warm_steps
-    R = max(1, math.ceil(args.min_ms / max(K * est_step, 1e-6)))
-    if world > 1:
-        t = torch.tensor([R], device=dev); dist.all_reduce(t, op=dist.ReduceOp.MAX); R = int(t.item())
-    n_timed = K * R
     if use_graphs and n_timed % P:
-        tail_graphs_for(n_timed % P)
-    timed(min(n_timed, 2 * P))   # one more untimed run of the exact graph set
+        tail_graphs_for(n_timed % P)   # capture outside any timed region
+    timed(warm_steps)
+    if n_timed % P:
+        timed(n_timed % P)   # the partial rotation's graphs run once before they are timed
 
     trials, kernel_mhz = [], []
     with ClockSampler(local_rank, period_s=0.010) as clk:
@@ -557,6 +585,13 @@ def run_b200(args, cfg: dict, rank: int, local_rank: int, world: int) -> None:
             kernel_mhz.append(round(statistics.median(e.last_pass_sm_clock() for e in engines), 1))
     for e in engines:
         e.check_indices()
+    if args.dump_outputs and rank == 0:
+        # the last timed step ran pool entry (K - 1) mod P; at N > 1 its assembled [world, block] rows are what every
+        # rank's caller receives
+        blocks = pool[(n_timed - 1) % P][2]["assembled"].view(max(world, 1), blk_bytes)
+        f32 = [b[B * 2 * E:].view(torch.float32).view(3, B) for b in blocks]
+        dump_outputs(args.dump_outputs, {"gen_out": torch.cat([b[:B * 2 * E].view(torch.bfloat16).view(B, E) for b in blocks]),
+                                         **{name: torch.cat([x[j] for x in f32]) for j, name in enumerate(OUTPUT_NAMES[1:])}})
     ms_med, ms_best = statistics.median(trials), min(trials)
     value = Bg * n_timed / (ms_med * 1e-3)
     gpu_launches = int(round(launches_per_step * n_timed))
@@ -669,13 +704,14 @@ def run_b200(args, cfg: dict, rank: int, local_rank: int, world: int) -> None:
     ach = flops[dom] / (kinds[dom]["ms_per_launch"] * 1e-3) / 1e12
     step_tflops = FLOP_SAMPLE * value / world / 1e12
     # Denominator (B200_PROFILING.md: "the burst figure for a kernel timed alone, the sustained one for a kernel timed
-    # inside a long step"): the timed region is >= 50 ms of back-to-back passes, repeated; when NVML reports the power
-    # cap during it (SM clocks below the maximum) the sustained cuBLAS figure is the like-for-like peak, otherwise the
-    # burst one.  Both fractions are always printed.
+    # inside a long step"): the timed region is `steps` back-to-back passes, its length follows --steps.  When it lasts
+    # at least SUSTAINED_MIN_MS and NVML reports the power cap during it (SM clocks below the maximum), the sustained
+    # cuBLAS figure is the like-for-like peak; a shorter region runs mostly before the cap lowers the clock, so the
+    # burst figure is.  Both fractions are always printed, and peak_source says which one `frac` uses.
     clock_summary = clk.summary()
     clock_summary["sm_mhz_in_kernel_by_trial"] = kernel_mhz   # clock64 / globaltimer over a pass's lifetime (pbg_last_pass_sm_clock)
     capped = "sw_power_cap" in (clock_summary.get("reasons") or [])
-    use_sustained = capped and ms_med >= 25.0
+    use_sustained = capped and ms_med >= SUSTAINED_MIN_MS
     peak = peaks["bf16_sustained"] if use_sustained else peaks["bf16_burst"]
     ctas_avg = sum((w if w > 0 else num_sms) for w in widths) / len(widths)
     share = ctas_avg / num_sms
@@ -690,7 +726,8 @@ def run_b200(args, cfg: dict, rank: int, local_rank: int, world: int) -> None:
                 "frac": step_tflops / peak, "traffic": traffic, "traffic_source": traffic_src,
                 "peak_source": peaks["source"] + (", SUSTAINED figure (cuBLAS bf16 back to back for seconds under the power cap): this "
                                                   f"timed region is {ms_med:.0f} ms x {len(trials)} trials and NVML reported sw_power_cap during it"
-                                                  if use_sustained else ", burst figure (cuBLAS bf16 8192^3, best of 10)"),
+                                                  if use_sustained else f", burst figure (cuBLAS bf16 8192^3, best of 10): this timed "
+                                                  f"region is {ms_med:.1f} ms" + ("" if capped else " and NVML reported no sw_power_cap")),
                 "frac_of_burst": step_tflops / peaks["bf16_burst"], "frac_of_sustained": step_tflops / peaks["bf16_sustained"],
                 "best_trial_frac_of_burst": FLOP_SAMPLE * (Bg * n_timed / (ms_best * 1e-3)) / world / 1e12 / peaks["bf16_burst"],
                 "note": f"achieved = algorithmic flops per sample x measured throughput of the timed region (median "
@@ -722,11 +759,12 @@ def run_b200(args, cfg: dict, rank: int, local_rank: int, world: int) -> None:
             "metric": METRIC, "value": value, "unit": "samples/s", "n_gpus": world, "steps": K, "warmup": W,
             "ms_per_step": ms_med / n_timed, "higher_is_better": True, "scaling": "weak", "vs_baseline": None,
             "dtype": "bf16", "data": "synthetic",
-            "repeats": R, "trials_ms": [round(x, 4) for x in trials], "best": Bg * n_timed / (ms_best * 1e-3),
+            "trials_ms": [round(x, 4) for x in trials], "best": Bg * n_timed / (ms_best * 1e-3),
             "config": {"workload": workload_name(cfg, B, world, "bf16"), "global_batch": Bg, "parallelism": f"dp{world}",
-                       "timed_region": f"{K} steps x {R} repeats = {n_timed} passes in one CUDA-event pair (>= {args.min_ms:.0f} ms), "
-                                       f"median of {len(trials)} trials; warm-up ran {warm_steps} + {min(n_timed, 2 * P)} steps "
-                                       f"after every pool entry had executed once",
+                       "timed_region": f"{n_timed} passes in one CUDA-event pair ({ms_med:.1f} ms"
+                                       + (", short: includes the lanes' ramp and tail" if ms_med < SUSTAINED_MIN_MS else "")
+                                       + f"), median of {len(trials)} trials; warm-up ran "
+                                       f"{warm_steps} + {n_timed % P} steps after every pool entry had executed once",
                        "l2": f"inputs rotate over {P} distinct pre-staged batches ({P * per_batch / 2**20:.0f} MiB "
                              f"> 126 MiB L2); no flush", "cuda_graphs": bool(use_graphs),
                        "lanes": S, "ctas_per_pass": [w if w > 0 else num_sms for w in widths[:min(S, 3)]],
@@ -750,7 +788,7 @@ def run_b200(args, cfg: dict, rank: int, local_rank: int, world: int) -> None:
 def main() -> None:
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=100)
+    ap.add_argument("--steps", type=int, default=2000, help="timed passes per trial (the default is a region of ~50 ms)")
     ap.add_argument("--warmup", type=int, default=20)
     ap.add_argument("--impl", choices=["b200", "reference"], default="b200")
     ap.add_argument("--config", choices=sorted(CONFIGS), default="base")
@@ -765,11 +803,14 @@ def main() -> None:
     ap.add_argument("--e2e-threads", type=int, default=0, help="host threads of the e2e leg (0: one per lane)")
     ap.add_argument("--e2e-min-s", type=float, default=0.4, help="the e2e leg runs at least this long (and >= --steps calls)")
     ap.add_argument("--ctas", type=int, default=0, help="SMs per pass (0: 50 / 50 / 48 of 148, whole CTA pairs)")
-    ap.add_argument("--min-ms", type=float, default=50.0, help="minimum length of one timed region (sets `repeats`)")
-    ap.add_argument("--trials", type=int, default=5)
+    ap.add_argument("--trials", type=int, default=5, help="timed regions of --steps steps each; the median is the headline")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-library-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write what the last timed step returned to DIR/<name>.npy (float32, at most 64 MiB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        raise SystemExit("bench.py: --steps must be >= 1")
     cfg = CONFIGS[args.config]
     if args.batch <= 0:
         args.batch = cfg["batch"]

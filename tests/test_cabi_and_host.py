@@ -143,14 +143,19 @@ print("OK", rank)
 """
 
 
+def _free_port() -> int:
+    import socket
+    with socket.socket() as s:
+        s.bind(("127.0.0.1", 0))
+        return s.getsockname()[1]
+
+
 def test_batch_sharding_plus_allgather_world_size_2_gloo(tmp_path):
     """The N > 1 path on CPU: 2 gloo ranks shard by batch index, run their shard, all-gather, compare with the
     unsharded pass."""
     script = tmp_path / "worker.py"
     script.write_text(_GLOO_WORKER)
-    import socket
-    with socket.socket() as s:
-        s.bind(("127.0.0.1", 0)); port = s.getsockname()[1]
+    port = _free_port()
     procs = []
     for r in range(2):
         env = dict(os.environ, RANK=str(r), WORLD_SIZE="2", MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port),
@@ -162,14 +167,48 @@ def test_batch_sharding_plus_allgather_world_size_2_gloo(tmp_path):
         assert p.returncode == 0 and f"OK {r}" in o, o
 
 
-def test_bench_reference_arm_prints_one_json_line():
+def _bench_module():
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench_mod", str(ROOT / "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    return bench
+
+
+def test_bench_reference_arm_prints_one_json_line(tmp_path):
     import json
+    import numpy as np
     out = subprocess.run([sys.executable, str(ROOT / "bench.py"), "--impl", "reference", "--steps", "2", "--warmup", "3",
-                          "--batch", "256"], capture_output=True, text=True, timeout=300)
+                          "--batch", "256", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=300)
     assert out.returncode == 0, out.stderr
     line = json.loads(out.stdout.strip().splitlines()[-1])
     assert line["impl"] == "reference" and line["unit"] == "samples/s" and line["value"] > 0
     assert line["cpu_baseline"]["kind"] == "port" and line["e2e"]["h2d_bytes_per_step"] == 0
+    # --dump-outputs: what the last timed step returned, float32, one row per triplet
+    shapes = {"gen_out": (256, 128), "gen_scores": (256,), "logits": (256,), "probs": (256,)}
+    assert sorted(p.name for p in tmp_path.iterdir()) == sorted(f"{k}.npy" for k in shapes)
+    for k, shape in shapes.items():
+        a = np.load(tmp_path / f"{k}.npy")
+        assert a.dtype == np.float32 and a.shape == shape and np.isfinite(a).all(), k
+    assert np.allclose(np.load(tmp_path / "probs.npy"), 1 / (1 + np.exp(-np.load(tmp_path / "logits.npy"))), atol=1e-6)
+
+
+def test_bench_dump_outputs_keeps_a_seeded_sample_under_the_limit(tmp_path):
+    import numpy as np
+    bench = _bench_module()
+    bench.DUMP_MAX_BYTES = 3000
+    g = torch.Generator().manual_seed(5)
+    arrays = {"gen_out": torch.randn(100, 8, generator=g), "logits": torch.randn(100, generator=g)}
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), arrays)
+    files = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert files == ["gen_out.npy", "logits.npy", "rows.npy"]
+    assert sum((tmp_path / "a" / f).stat().st_size for f in files) <= 3000
+    rows = np.load(tmp_path / "a" / "rows.npy")
+    assert rows.dtype == np.float64 and 0 < len(rows) < 100 and (np.diff(rows) > 0).all()
+    for f in files:
+        assert np.array_equal(np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)), f   # the same sample every time
+    assert np.array_equal(np.load(tmp_path / "a" / "gen_out.npy"), arrays["gen_out"].numpy()[rows.astype(int)])
 
 
 @pytest.mark.skipif(torch.cuda.is_available(), reason="checks the no-GPU failure mode")
@@ -183,7 +222,7 @@ def test_bench_reference_arm_under_torchrun_prints_one_line_from_rank_0():
     """N > 1: the driver launches the reference arm like the product arm; rank 0 alone measures and prints."""
     import json
     out = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--nnodes=1", "--nproc-per-node", "2",
-                          "--master-addr", "127.0.0.1", "--master-port", "29611", str(ROOT / "bench.py"), "--impl",
+                          "--master-addr", "127.0.0.1", "--master-port", str(_free_port()), str(ROOT / "bench.py"), "--impl",
                           "reference", "--gpus", "2", "--steps", "2", "--warmup", "3", "--batch", "256"],
                          capture_output=True, text=True, timeout=600)
     assert out.returncode == 0, out.stderr[-2000:]
@@ -208,10 +247,7 @@ def test_top_k_is_validated_on_the_host_before_anything_is_launched():
 
 def test_bench_flop_and_config_table_match_the_survey():
     """bench.py's algorithmic flop counts are SURVEY.md 8d's (2*K*N per Linear) for both BASELINE model shapes."""
-    import importlib.util
-    spec = importlib.util.spec_from_file_location("bench_mod", str(ROOT / "bench.py"))
-    bench = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(bench)
+    bench = _bench_module()
     assert bench.flops_per_sample(128, 64, 1024) == (3014656, 1836032)
     assert bench.flops_per_sample(256, 64, 4096) == (40370176, 23072768)
     assert bench.CONFIGS["base"]["batch"] == 4096 and bench.CONFIGS["wide"]["batch"] == 1024

@@ -659,3 +659,38 @@ def test_host_entry_points_packed_and_per_buffer(engine, dev_tables, synth, dev,
     assert torch.equal(gen.bfloat16(), ref["gen_out"].cpu())   # the host form returns fp32 rows of the same values
     with pytest.raises(ValueError):
         engine.score_triplets_host_packed(*dev_tables, blk[:-8], hb, B)
+
+
+def test_bench_dump_outputs_are_the_last_timed_steps_results(synth, dev, tmp_path):
+    """bench.py --dump-outputs on the B200 arm: the last of K timed steps ran pool entry K - 1 (K below the pool size);
+    its dumped rows equal, bit for bit, a direct fused pass over that entry's seeded inputs."""
+    import importlib.util
+    import subprocess
+    import sys
+    from pathlib import Path
+    import numpy as np
+    import modular_prot_b_gan as m
+    root = Path(__file__).resolve().parent.parent
+    K = 20
+    out = subprocess.run([sys.executable, str(root / "bench.py"), "--steps", str(K), "--warmup", "3", "--trials", "1",
+                          "--no-cpu-baseline", "--no-library-baseline", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-3000:]
+    spec = importlib.util.spec_from_file_location("bench_mod", str(root / "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    cfg = bench.CONFIGS["base"]
+    B = cfg["batch"]
+    G, D = bench.make_models(cfg, m.ModularGenerator, m.ModularDiscriminator)
+    eng = m.make_fused_engine(G.to(dev), D.to(dev))
+    node_emb, rel_w = (t.to(dev) for t in synth.make_tables(bench.NUM_ENTITIES, bench.NUM_RELATIONS, cfg["E"]))
+    trip = synth.make_triplets(B, bench.NUM_ENTITIES, bench.NUM_RELATIONS, seed=4321 + K - 1).to(dev)
+    z = synth.make_latents(B, cfg["Z"], seed=1234 + K - 1).to(dev)
+    ref = eng.score_triplets(node_emb, rel_w, trip, z, want_gen_out=True, want_gen_scores=True, want_disc=True,
+                             precision="bf16", out_dtype=torch.bfloat16)
+    torch.cuda.synchronize()
+    assert sorted(p.name for p in tmp_path.iterdir()) == ["gen_out.npy", "gen_scores.npy", "logits.npy", "probs.npy"]
+    for k in ("gen_out", "gen_scores", "logits", "probs"):
+        got = np.load(tmp_path / f"{k}.npy")
+        assert got.dtype == np.float32, k
+        assert np.array_equal(got, ref[k].float().cpu().numpy()), k
