@@ -82,7 +82,8 @@ int pbg_load_discriminator(pbg_ctx* ctx, const float* packed_host, size_t n_floa
 
 /* Replaces `self.generator(h_emb, r_emb)` (pro_b_gan_infer.py:143, :201).
  * h, r: [B,E] fp32; z: [B,Z] fp32 latents (the reference's forward takes no noise argument;
- * the host module draws z from its seeded CPU generator and passes it here).
+ * the host module draws z from its seeded CPU generator and passes it here; NULL draws from the ctx's latent
+ * stream, see pbg_set_latent_stream).
  * out: [B,E] of `out_dtype`.  tanh output. */
 int pbg_generator_forward(pbg_ctx* ctx, const float* h, const float* r, const float* z, void* out,
                           int64_t B, int precision, int out_dtype, void* stream);
@@ -140,6 +141,42 @@ int pbg_score_triplets_host_packed(pbg_ctx* ctx, const float* node_emb, int64_t 
                                    int64_t R, const void* in_block_host, float* out_block_host, int64_t B,
                                    int precision);
 
+/* Device latents.  torch.randn((rows, Z), device='cuda', generator=g) is fully set by g's Philox (seed, offset), the
+ * launch geometry of torch's normal_ and curand_normal4: element e of a draw of numel = rows * Z elements comes from
+ * thread t = e % T, round r = e / 4T, component j = (e / T) % 4 with T = 256 * min(SMs * max_threads_per_SM / 256,
+ * ceil(numel / 256)), and the draw advances the offset by ((numel - 1) / 4T + 1) * 4.  These calls reproduce that stream
+ * bit for bit on the device (numel < 2^31; larger draws are PBG_ERR_UNSUPPORTED).  The CPU stream the host modules
+ * draw from by default (mt19937) is a different stream.
+ *
+ * pbg_draw_latents writes rows [row_begin, row_begin + rows) of a [total_rows, Z] draw at (seed, offset) to z_out
+ * [rows, Z] fp32, stream-ordered; ranges that tile [0, total_rows) concatenate to the whole draw, so a batch-sharded
+ * job can draw its own shard.  *offset_after (if non-NULL) receives the offset after the whole draw.  Stateless. */
+int pbg_draw_latents(pbg_ctx* ctx, uint64_t seed, uint64_t offset, int64_t total_rows, int64_t row_begin,
+                     int64_t rows, float* z_out, uint64_t* offset_after, void* stream);
+
+/* The ctx's latent stream (off by default).  While it is enabled, every entry point that runs the generator accepts
+ * z == NULL (pbg_generator_forward[_gather], pbg_score_triplets, pbg_score_triplets_host with z_host == NULL,
+ * pbg_stage_triplets, pbg_score_staged_stage_next with next_z == NULL) and draws the call's [B, Z] latents from
+ * (seed, offset), then advances the offset as torch would: a sequence of such calls sees what the same calls given
+ * z = torch.randn((B, Z), device='cuda', generator=g) see for a generator g at the same (seed, offset).
+ *   - a call of B > 65536 rows (processed in chunks) draws each chunk's rows of ONE [B, Z] draw;
+ *   - staged requests draw when they are staged (stream order = staging order); discriminator-only calls draw nothing;
+ *   - caller-supplied latents always win and leave the stream where it was;
+ *   - with the stream disabled, z == NULL is refused (PBG_ERR_INVALID) as before.
+ * The offset lives in device memory and each draw kernel advances it, so a CUDA graph captured over such calls draws
+ * fresh latents on every replay, as successive eager calls would; the seed is a launch argument and a graph keeps
+ * the one it was captured with.  Draws from one ctx's stream must be ordered among themselves (one stream, or
+ * events between an ingest and a compute stream), as the staging calls already are.  pbg_set_latent_stream
+ * synchronises the device; pbg_get_latent_stream synchronises `stream` and reads the current position. */
+int pbg_set_latent_stream(pbg_ctx* ctx, int enable, uint64_t seed, uint64_t offset);
+int pbg_get_latent_stream(pbg_ctx* ctx, uint64_t* seed, uint64_t* offset, void* stream);
+
+/* pbg_score_triplets_host_packed without latents on the wire: in-block = triplets int64 [B, 3] only (24 B per
+ * sample), out-block = [gen_scores | logits | probs] fp32 B each (12 B per sample); the latents come from the ctx's
+ * latent stream, which must be enabled (else PBG_ERR_INVALID).  Generator + discriminator both run.  Synchronous. */
+int pbg_score_triplets_host_ids(pbg_ctx* ctx, const float* node_emb, int64_t N, const float* rel_emb, int64_t R,
+                                const int64_t* triplets_host, float* out_block_host, int64_t B, int precision);
+
 /* Request staging -- the ingest / compute split of the same pass for callers that keep requests in flight.
  * pbg_score_triplets does gather -> layers in one launch, so the first tiles of every pass wait for its gather.
  * A server (or bench.py) that already holds the NEXT request's ids and latents on the device can stage it while the
@@ -152,7 +189,7 @@ int pbg_score_triplets_host_packed(pbg_ctx* ctx, const float* node_emb, int64_t 
  *       results as in pbg_score_triplets.  bf16 mode only.
  * Both are stream-ordered; the CALLER orders a slot's uses across the two streams (stage -> score -> next stage of the
  * same slot: two events, or one stream).  A ctx still runs one pass at a time.
- * pbg_reserve sizes the activation workspace (and `stage_slots` staging slots) for `rows` rows up front: buffers
+ * pbg_reserve sizes the activation and latent workspaces (and `stage_slots` staging slots) for `rows` rows up front: buffers
  * otherwise grow lazily with a device synchronisation, which is refused (PBG_ERR_INVALID) while the stream is being
  * captured into a CUDA graph. */
 int pbg_reserve(pbg_ctx* ctx, int64_t rows, int precision, int stage_slots);

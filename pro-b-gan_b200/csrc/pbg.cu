@@ -1,5 +1,6 @@
 // pbg.cu -- libpbg_b200.so: context, weight ingest, workspaces, TMA descriptors and the launch sequence behind
-// the C ABI declared in include/pbg.h.  Device code lives in gather.cuh / pass2_kernel.cuh / topk_kernel.cuh / gemm_f32.cuh.
+// the C ABI declared in include/pbg.h.  Device code lives in gather.cuh / pass2_kernel.cuh / topk_kernel.cuh / gemm_f32.cuh /
+// latent.cuh.
 //
 // HBM layout per ctx (sized lazily to the largest batch chunk seen, <= kMaxChunk rows):
 //   weights   : fp32 [out,in] + bias (parity mode) and bf16 [out_p, in_p] zero-padded to the tile grid + padded bias
@@ -34,6 +35,7 @@
 #include "topk_kernel.cuh"
 #include "index_rows.cuh"
 #include "json_out.cuh"
+#include "latent.cuh"
 
 using namespace pbg;
 
@@ -90,6 +92,7 @@ struct StageSlot {
   long long cap = 0;  // rows allocated
   void *xg0 = nullptr, *xd0 = nullptr;
   float* xt = nullptr;  // fp32 tail rows [cap, E] for the cosine epilogue
+  float* z = nullptr;   // fp32 latents [cap, Z] drawn from the ctx's latent stream when the request brings none
   CUtensorMap tm_xg0, tm_xd0;
   long long B = -1;     // rows of the staged request (-1: nothing staged)
   bool has_g = false, has_d = false;
@@ -108,6 +111,7 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t,
 struct pbg_ctx {
   pbg_dims dims{};
   int num_sms = 0;
+  int max_threads_sm = 0;   // with num_sms, sets torch's launch geometry that the latent draw reproduces
   bool g_loaded = false, d_loaded = false;
   int kg0 = 0, kg0p = 0, kd0 = 0, kd0p = 0, hgp = 0, hdp = 0, hd2 = 0, hd2p = 0, ep = 0, hmax = 0;
   Linear g[3], d[2];
@@ -127,6 +131,12 @@ struct pbg_ctx {
   float *st_z = nullptr, *st_gen = nullptr, *st_scores = nullptr, *st_logits = nullptr, *st_probs = nullptr;
   EncodeTiledFn encode = nullptr;
   TopkState tk;
+  // latent stream (pbg_set_latent_stream): generator calls without z draw from Philox (lat_seed, lat_st->offset)
+  bool lat_on = false;
+  unsigned long long lat_seed = 0;
+  LatentStream* lat_st = nullptr;   // device: the offset, advanced by each draw
+  long long lat_cap = 0;            // rows of lat_z
+  float* lat_z = nullptr;           // [lat_cap, Z] the drawn latents of the current chunk
   long long launches = 0;
   int launch_ctas = 0;  // pbg_set_launch_width; 0 = all SMs
   int discard = 1;      // pbg_set_workspace_discard (PBG_DISCARD sets the initial value)
@@ -239,7 +249,7 @@ int refuse_growth_in_capture(pbg_ctx* c, cudaStream_t s, const char* what) {
 }
 
 void free_stage(StageSlot& st) {
-  cudaFree(st.xg0); cudaFree(st.xd0); cudaFree(st.xt);
+  cudaFree(st.xg0); cudaFree(st.xd0); cudaFree(st.xt); cudaFree(st.z);
   st = StageSlot{};
 }
 
@@ -302,10 +312,58 @@ int ensure_stage(pbg_ctx* c, StageSlot& st, long long rows, cudaStream_t stream)
   PBG_CUDA(c, cudaMalloc(&st.xg0, es * cap * c->kg0p));
   PBG_CUDA(c, cudaMalloc(&st.xd0, es * cap * c->kd0p));
   PBG_CUDA(c, cudaMalloc(&st.xt, sizeof(float) * cap * c->dims.embed_dim));
+  PBG_CUDA(c, cudaMalloc(&st.z, sizeof(float) * cap * c->dims.noise_dim));
   PBG_TRY(make_tmap(c, &st.tm_xg0, st.xg0, cap, c->kg0p, kBlockM));
   PBG_TRY(make_tmap(c, &st.tm_xd0, st.xd0, cap, c->kd0p, kBlockM));
   st.cap = cap;
   return PBG_OK;
+}
+
+int ensure_latents(pbg_ctx* c, long long rows, cudaStream_t stream) {
+  if (c->lat_cap >= rows) return PBG_OK;
+  PBG_TRY(refuse_growth_in_capture(c, stream, "the latent workspace"));
+  long long cap = 1024;
+  while (cap < rows) cap *= 2;
+  cap = std::min(cap, kMaxChunk);
+  PBG_CUDA(c, cudaDeviceSynchronize());  // nothing may still be reading the old buffer
+  cudaFree(c->lat_z); c->lat_z = nullptr; c->lat_cap = 0;
+  PBG_CUDA(c, cudaMalloc(&c->lat_z, sizeof(float) * cap * c->dims.noise_dim));
+  c->lat_cap = cap;
+  return PBG_OK;
+}
+
+// torch splits a tensor of 2^31 elements or more into several launches, each with its own geometry and offset
+int check_draw_size(pbg_ctx* c, long long total_rows) {
+  if (total_rows < 1) return fail(c, PBG_ERR_INVALID, "latent draw: total_rows must be positive");
+  if (total_rows > 0x7fffffffll / c->dims.noise_dim)
+    return fail(c, PBG_ERR_UNSUPPORTED, "latent draw: %lld x %d elements is above the 2^31 - 1 of one torch launch",
+                total_rows, c->dims.noise_dim);
+  return PBG_OK;
+}
+
+// Rows [row_begin, row_begin + rows) of a [total_rows, Z] draw (latent.cuh) into out, at Philox (seed, offset) --
+// or at (seed, st->offset) when st is given, advancing st->offset past the whole draw when `advance`.
+int launch_draw(pbg_ctx* c, unsigned long long seed, unsigned long long offset, LatentStream* st, bool advance,
+                long long total_rows, long long row_begin, long long rows, float* out, cudaStream_t s) {
+  if (rows <= 0) return PBG_OK;
+  const long long Z = c->dims.noise_dim;
+  const LatentGeometry g = latent_geometry(total_rows * Z, c->num_sms, c->max_threads_sm);
+  LatentParams p{};
+  p.seed = seed; p.offset = offset; p.st = st; p.advance = advance ? 1 : 0; p.inc = g.inc; p.T = g.T;
+  p.e_begin = row_begin * Z; p.e_end = (row_begin + rows) * Z; p.out = out;
+  const long long r_lo = p.e_begin / (4 * g.T), r_hi = (p.e_end - 1) / (4 * g.T);
+  p.slot_begin = r_lo * g.T;
+  const long long blocks = (r_hi - r_lo + 1) * g.T / kLatentThreads;   // T is a multiple of the block
+  { LaunchScope ls(c, PBG_K_OTHER, s);
+    latent_draw_kernel<<<static_cast<unsigned>(blocks), kLatentThreads, 0, s>>>(p); }
+  PBG_CUDA(c, cudaGetLastError());
+  return PBG_OK;
+}
+
+// Draw a request's latents from the ctx's stream (staging: the whole request at once).
+int draw_stream(pbg_ctx* c, long long B, float* out, cudaStream_t s) {
+  PBG_TRY(check_draw_size(c, B));
+  return launch_draw(c, c->lat_seed, 0, c->lat_st, true, B, 0, B, out, s);
 }
 
 template <int ACT>
@@ -337,6 +395,7 @@ struct Pass {
   const long long *heads = nullptr, *rels = nullptr, *tails = nullptr;
   long long hs = 1, rs = 1, ts = 1;
   const float *h = nullptr, *r = nullptr, *t = nullptr, *z = nullptr;
+  bool draw_z = false;   // z == nullptr with the latent stream on: each chunk draws its rows of ONE draw over B
   void* gen_out = nullptr; int out_dtype = PBG_DT_F32;
   float *gen_scores = nullptr, *logits = nullptr, *probs = nullptr;
   bool run_g = false, run_d = false;
@@ -356,6 +415,10 @@ int run_chunk(pbg_ctx* c, const Pass& a, long long off, long long rows) {
   gp.tails = a.tails ? a.tails + off * a.ts : nullptr; gp.tail_stride = a.ts;
   gp.h = a.h ? a.h + off * E : nullptr; gp.r = a.r ? a.r + off * E : nullptr; gp.t = a.t ? a.t + off * E : nullptr;
   gp.z = a.z ? a.z + off * Z : nullptr;
+  if (a.draw_z) {
+    PBG_TRY(launch_draw(c, c->lat_seed, 0, c->lat_st, off + rows == a.B, a.B, off, rows, c->lat_z, s));
+    gp.z = c->lat_z;
+  }
   gp.xg = a.run_g ? w.xg0 : nullptr; gp.ldg = bf ? c->kg0p : c->kg0;
   gp.xd = a.run_d ? w.xd0 : nullptr; gp.ldd = bf ? c->kd0p : c->kd0;
   gp.B = rows; gp.err_flag = c->err_flag;
@@ -595,13 +658,15 @@ int launch_pass2(pbg_ctx* c, Workspace& w, const Pass& a, const GatherParams& gp
   return PBG_OK;
 }
 
-int run_pass(pbg_ctx* c, const Pass& a) {
+int run_pass(pbg_ctx* c, Pass a) {
   if (!c) return PBG_ERR_INVALID;
   if (a.B < 0) return fail(c, PBG_ERR_INVALID, "negative batch");
   if (a.prec != PBG_PREC_F32 && a.prec != PBG_PREC_BF16) return fail(c, PBG_ERR_INVALID, "unknown precision %d", a.prec);
   if (a.run_g && !c->g_loaded) return fail(c, PBG_ERR_NOT_LOADED, "generator weights not loaded");
   if (a.run_d && !c->d_loaded) return fail(c, PBG_ERR_NOT_LOADED, "discriminator weights not loaded");
-  if (a.run_g && a.z == nullptr) return fail(c, PBG_ERR_INVALID, "generator needs latents z");
+  if (a.run_g && a.z == nullptr && !c->lat_on) return fail(c, PBG_ERR_INVALID, "generator needs latents z");
+  a.draw_z = a.run_g && a.z == nullptr && a.B > 0;
+  if (a.draw_z) PBG_TRY(check_draw_size(c, a.B));
   if (a.run_g && a.gen_out && a.prec == PBG_PREC_F32 && a.out_dtype != PBG_DT_F32)
     return fail(c, PBG_ERR_INVALID, "fp32 mode writes fp32 output");
   if (a.gen_scores && a.tails == nullptr) return fail(c, PBG_ERR_INVALID, "gen_scores needs tail ids");
@@ -609,6 +674,7 @@ int run_pass(pbg_ctx* c, const Pass& a) {
   PBG_CUDA(c, cudaSetDevice(c->dims.device));
   const long long chunk = std::min(a.B, kMaxChunk);
   PBG_TRY(ensure_ws(c, a.prec, chunk, a.stream));
+  if (a.draw_z) PBG_TRY(ensure_latents(c, chunk, a.stream));
   for (long long off = 0; off < a.B; off += chunk) PBG_TRY(run_chunk(c, a, off, std::min(chunk, a.B - off)));
   return PBG_OK;
 }
@@ -941,6 +1007,7 @@ int pbg_create(pbg_ctx** out, const pbg_dims* dims) {
   if (!c) return fail(nullptr, PBG_ERR_NOMEM, "out of host memory");
   c->dims = *dims;
   c->num_sms = prop.multiProcessorCount;
+  c->max_threads_sm = prop.maxThreadsPerMultiProcessor;
   if (const char* e = getenv("PBG_DISCARD")) c->discard = atoi(e) != 0;
   if (const char* e = getenv("PBG_HOST_SYNC")) c->host_block = strcmp(e, "block") == 0;
   c->kg0 = 2 * E + Z; c->kg0p = round_up(c->kg0, kBlockK);
@@ -961,7 +1028,9 @@ int pbg_create(pbg_ctx** out, const pbg_dims* dims) {
   if (cudaStreamCreateWithFlags(&c->own_stream, cudaStreamNonBlocking) != cudaSuccess ||
       cudaMalloc(&c->err_flag, sizeof(int)) != cudaSuccess ||
       cudaMemset(c->err_flag, 0, sizeof(int)) != cudaSuccess ||
-      cudaMallocHost(&c->err_flag_host, sizeof(int)) != cudaSuccess) {
+      cudaMallocHost(&c->err_flag_host, sizeof(int)) != cudaSuccess ||
+      cudaMalloc(&c->lat_st, sizeof(LatentStream)) != cudaSuccess ||
+      cudaMemset(c->lat_st, 0, sizeof(LatentStream)) != cudaSuccess) {
     c->err = std::string("ctx allocation failed: ") + cudaGetErrorString(cudaGetLastError());
     return bail(PBG_ERR_CUDA);
   }
@@ -980,6 +1049,7 @@ void pbg_destroy(pbg_ctx* c) {
   free_ws(c->ws_bf16); free_ws(c->ws_f32);
   free_stage(c->stage[0]); free_stage(c->stage[1]);
   cudaFree(c->err_flag); cudaFree(c->trace);
+  cudaFree(c->lat_st); cudaFree(c->lat_z);
   cudaFree(c->tk.tn); cudaFree(c->tk.inv_t); cudaFree(c->tk.qn); cudaFree(c->tk.inv_q);
   cudaFree(c->tk.cand_grp); cudaFree(c->tk.cand_mask); cudaFree(c->tk.cand_cnt); cudaFree(c->tk.flag);
   cudaFree(c->tk.samp_keys); cudaFree(c->tk.tau); cudaFree(c->tk.score_buf);
@@ -1094,7 +1164,47 @@ int pbg_reserve(pbg_ctx* c, int64_t rows, int precision, int stage_slots) {
   PBG_CUDA(c, cudaSetDevice(c->dims.device));
   const long long chunk = std::min<long long>(rows, kMaxChunk);
   PBG_TRY(ensure_ws(c, precision, chunk, nullptr));
+  PBG_TRY(ensure_latents(c, chunk, nullptr));
   for (int i = 0; i < stage_slots; ++i) PBG_TRY(ensure_stage(c, c->stage[i], chunk, nullptr));
+  return PBG_OK;
+}
+
+int pbg_draw_latents(pbg_ctx* c, uint64_t seed, uint64_t offset, int64_t total_rows, int64_t row_begin, int64_t rows,
+                     float* z_out, uint64_t* offset_after, void* stream) {
+  if (!c) return PBG_ERR_INVALID;
+  PBG_TRY(check_draw_size(c, total_rows));
+  if (row_begin < 0 || rows < 0 || row_begin + rows > total_rows)
+    return fail(c, PBG_ERR_INVALID, "latent draw: rows [%lld, %lld) outside the %lld of the draw", (long long)row_begin,
+                (long long)(row_begin + rows), (long long)total_rows);
+  if (rows > 0 && !z_out) return fail(c, PBG_ERR_INVALID, "null tensor");
+  if (offset % 4) return fail(c, PBG_ERR_INVALID, "latent draw: the Philox offset must be a multiple of 4, as torch's");
+  PBG_CUDA(c, cudaSetDevice(c->dims.device));
+  PBG_TRY(launch_draw(c, seed, offset, nullptr, false, total_rows, row_begin, rows, z_out, (cudaStream_t)stream));
+  if (offset_after)
+    *offset_after = offset + latent_geometry(total_rows * c->dims.noise_dim, c->num_sms, c->max_threads_sm).inc;
+  return PBG_OK;
+}
+
+int pbg_set_latent_stream(pbg_ctx* c, int enable, uint64_t seed, uint64_t offset) {
+  if (!c) return PBG_ERR_INVALID;
+  if (offset % 4) return fail(c, PBG_ERR_INVALID, "latent stream: the Philox offset must be a multiple of 4, as torch's");
+  PBG_CUDA(c, cudaSetDevice(c->dims.device));
+  PBG_CUDA(c, cudaDeviceSynchronize());   // no draw of the ctx may still be reading or advancing the offset
+  const LatentStream st{offset, 0u};
+  PBG_CUDA(c, cudaMemcpy(c->lat_st, &st, sizeof st, cudaMemcpyHostToDevice));
+  c->lat_on = enable != 0;
+  c->lat_seed = seed;
+  return PBG_OK;
+}
+
+int pbg_get_latent_stream(pbg_ctx* c, uint64_t* seed, uint64_t* offset, void* stream) {
+  if (!c || !seed || !offset) return PBG_ERR_INVALID;
+  PBG_CUDA(c, cudaSetDevice(c->dims.device));
+  LatentStream st{};
+  PBG_CUDA(c, cudaMemcpyAsync(&st, c->lat_st, sizeof st, cudaMemcpyDeviceToHost, (cudaStream_t)stream));
+  PBG_CUDA(c, cudaStreamSynchronize((cudaStream_t)stream));
+  *seed = c->lat_seed;
+  *offset = st.offset;
   return PBG_OK;
 }
 
@@ -1107,11 +1217,15 @@ int pbg_stage_triplets(pbg_ctx* c, int slot, const float* node_emb, int64_t N, c
   if (!want_gen && !want_disc) return fail(c, PBG_ERR_INVALID, "stage: nothing to stage");
   if (want_gen && !c->g_loaded) return fail(c, PBG_ERR_NOT_LOADED, "generator weights not loaded");
   if (want_disc && !c->d_loaded) return fail(c, PBG_ERR_NOT_LOADED, "discriminator weights not loaded");
-  if (want_gen && !z) return fail(c, PBG_ERR_INVALID, "generator needs latents z");
+  if (want_gen && !z && !c->lat_on) return fail(c, PBG_ERR_INVALID, "generator needs latents z");
   PBG_CUDA(c, cudaSetDevice(c->dims.device));
   cudaStream_t s = (cudaStream_t)stream;
   StageSlot& st = c->stage[slot];
   PBG_TRY(ensure_stage(c, st, B, s));
+  if (want_gen && !z) {   // the request's latents from the ctx's stream, in staging order
+    PBG_TRY(draw_stream(c, B, st.z, s));
+    z = st.z;
+  }
   const long long* t = (const long long*)triplets;
   StageParams sp{};
   GatherParams& gp = sp.g;
@@ -1166,11 +1280,15 @@ int pbg_score_staged_stage_next(pbg_ctx* c, int slot, void* gen_out, int out_dty
   if (a.run_g && !st.has_g) return fail(c, PBG_ERR_INVALID, "score_staged: slot %d holds no generator operands", slot);
   if (a.run_d && !st.has_d) return fail(c, PBG_ERR_INVALID, "score_staged: slot %d holds no discriminator operands", slot);
   if (!a.run_g && !a.run_d) return fail(c, PBG_ERR_INVALID, "score_staged_stage_next: no result requested");
-  if (a.run_g && !next_z) return fail(c, PBG_ERR_INVALID, "generator needs latents z");
+  if (a.run_g && !next_z && !c->lat_on) return fail(c, PBG_ERR_INVALID, "generator needs latents z");
   a.B = st.B; a.prec = PBG_PREC_BF16; a.stream = (cudaStream_t)stream;
   PBG_CUDA(c, cudaSetDevice(c->dims.device));
   PBG_TRY(ensure_ws(c, PBG_PREC_BF16, st.B, a.stream));
   PBG_TRY(ensure_stage(c, nx, next_B, a.stream));
+  if (a.run_g && !next_z) {   // drawn now, ahead of the pass that gathers it: stream order is staging order
+    PBG_TRY(draw_stream(c, next_B, nx.z, a.stream));
+    next_z = nx.z;
+  }
   // the next request gets the operands this pass produces results for (same models in flight)
   const long long* t = reinterpret_cast<const long long*>(next_triplets);
   GatherParams gp{};
@@ -1313,7 +1431,7 @@ int score_host(pbg_ctx* c, const float* node_emb, int64_t N, const float* rel_em
   if (B == 0) return PBG_OK;
   if (!triplets_host) return fail(c, PBG_ERR_INVALID, "null triplets");
   const bool run_g = gen_out_host || gen_scores_host;
-  if (run_g && !z_host) return fail(c, PBG_ERR_INVALID, "generator needs latents z");
+  if (run_g && !z_host && !c->lat_on) return fail(c, PBG_ERR_INVALID, "generator needs latents z");
   PBG_CUDA(c, cudaSetDevice(c->dims.device));
   const int E = c->dims.embed_dim, Z = c->dims.noise_dim;
   if (c->host_cap < B) {
@@ -1339,14 +1457,14 @@ int score_host(pbg_ctx* c, const float* node_emb, int64_t N, const float* rel_em
   cudaStream_t s = c->own_stream;
   // every DMA operation costs a few microseconds of set-up beside its bytes (six of them were a third of a 4096-triplet
   // call): the packed form moves [triplets | z] and [scores | logits | probs] in one copy each
-  const bool one_h2d = packed && reinterpret_cast<char*>(c->st_z) == reinterpret_cast<char*>(c->st_trip) + sizeof(long long) * 3 * B;
+  const bool one_h2d = packed && z_host && reinterpret_cast<char*>(c->st_z) == reinterpret_cast<char*>(c->st_trip) + sizeof(long long) * 3 * B;
   if (one_h2d) {
     PBG_CUDA(c, cudaMemcpyAsync(c->st_trip, triplets_host, sizeof(long long) * 3 * B + sizeof(float) * Z * B, cudaMemcpyHostToDevice, s));
   } else {
     PBG_CUDA(c, cudaMemcpyAsync(c->st_trip, triplets_host, sizeof(long long) * 3 * B, cudaMemcpyHostToDevice, s));
-    if (run_g) PBG_CUDA(c, cudaMemcpyAsync(c->st_z, z_host, sizeof(float) * Z * B, cudaMemcpyHostToDevice, s));
+    if (run_g && z_host) PBG_CUDA(c, cudaMemcpyAsync(c->st_z, z_host, sizeof(float) * Z * B, cudaMemcpyHostToDevice, s));
   }
-  PBG_TRY(pbg_score_triplets(c, node_emb, N, rel_emb, R, (const int64_t*)c->st_trip, run_g ? c->st_z : nullptr,
+  PBG_TRY(pbg_score_triplets(c, node_emb, N, rel_emb, R, (const int64_t*)c->st_trip, run_g && z_host ? c->st_z : nullptr,
                              gen_out_host ? c->st_gen : nullptr, PBG_DT_F32, gen_scores_host ? c->st_scores : nullptr,
                              logits_host ? c->st_logits : nullptr, probs_host ? c->st_probs : nullptr, B, precision, s));
   if (packed) {
@@ -1376,6 +1494,15 @@ int pbg_score_triplets_host_packed(pbg_ctx* c, const float* node_emb, int64_t N,
   const float* z = reinterpret_cast<const float*>(static_cast<const char*>(in_block_host) + sizeof(long long) * 3 * B);
   return score_host(c, node_emb, N, rel_emb, R, trip, z, nullptr, out_block_host, out_block_host + B, out_block_host + 2 * B, B,
                     precision, true);
+}
+
+int pbg_score_triplets_host_ids(pbg_ctx* c, const float* node_emb, int64_t N, const float* rel_emb, int64_t R,
+                                const int64_t* triplets_host, float* out_block_host, int64_t B, int precision) {
+  if (!c) return PBG_ERR_INVALID;
+  if (!c->lat_on) return fail(c, PBG_ERR_INVALID, "score_triplets_host_ids draws the latents: enable the latent stream first");
+  if (B > 0 && (!triplets_host || !out_block_host)) return fail(c, PBG_ERR_INVALID, "null block");
+  return score_host(c, node_emb, N, rel_emb, R, triplets_host, nullptr, nullptr, out_block_host, out_block_host + B,
+                    out_block_host + 2 * B, B, precision, true);
 }
 
 }  // extern "C"

@@ -13,8 +13,13 @@ and handed to libpbg_b200.so, and every later forward is a C-ABI call.
 No CPU fallback and no second backend: a module left on the CPU, or a box without an sm_100 GPU, raises.
 Precision: ``PBG_PRECISION=bf16`` (default, tcgen05 tensor cores) or ``fp32`` (SIMT parity mode), or set the
 ``precision`` attribute on the module.
+Latents: ``PBG_LATENTS=cpu`` (default: the oracle's CPU mt19937 stream, copied to the device) or ``cuda`` (drawn on the
+device, bit for bit what ``torch.randn(..., device='cuda', generator=g)`` gives for g seeded LATENT_SEED), or set the
+generator's ``latent_source`` attribute.
 """
 from __future__ import annotations
+
+import os
 
 import torch
 import torch.nn as nn
@@ -63,7 +68,17 @@ class _CudaModule(nn.Module):
         raise NotImplementedError
 
 
+def latent_source(value: str | None = None) -> str:
+    """'cpu' or 'cuda': `value`, else the PBG_LATENTS env var, else 'cpu'."""
+    src = (value or os.environ.get("PBG_LATENTS", "cpu")).lower()
+    if src not in ("cpu", "cuda"):
+        raise ValueError(f"unknown latent source {src!r}; use 'cpu' or 'cuda'")
+    return src
+
+
 class ModularGenerator(_CudaModule):
+    latent_source: str | None = None   # None -> PBG_LATENTS env var -> 'cpu'
+
     def __init__(self, embed_dim: int, noise_dim: int, hidden_dim: int = DEFAULT_G_HIDDEN):
         super().__init__()
         self.embed_dim, self.noise_dim, self.hidden_dim = embed_dim, noise_dim, hidden_dim
@@ -79,11 +94,33 @@ class ModularGenerator(_CudaModule):
         )
         self._latent_gen = torch.Generator(device="cpu")
         self._latent_gen.manual_seed(LATENT_SEED)
+        self._latent_seed = LATENT_SEED
+        self._stream_engine: Engine | None = None   # the engine whose ctx holds the device latent stream
 
     def reseed(self, seed: int = LATENT_SEED) -> None:
+        """Restart the latent stream: the CPU generator, and the device stream (at Philox offset 0) with its next draw."""
         self._latent_gen.manual_seed(seed)
+        self._latent_seed = seed
+        self._stream_engine = None
+
+    def _device_stream(self) -> Engine:
+        """The engine, with its ctx's latent stream on; a rebuilt engine continues where the previous one stopped."""
+        eng = self._get_engine()
+        if self._stream_engine is not eng:
+            pos = self._stream_engine.latent_stream() if self._stream_engine is not None else (self._latent_seed, 0)
+            eng.set_latent_stream(True, *pos)
+            self._stream_engine = eng
+        return eng
 
     def sample_latent(self, batch: int) -> torch.Tensor:
+        if latent_source(self.latent_source) == "cuda":
+            eng = self._device_stream()
+            if batch == 0:
+                return torch.empty(0, self.noise_dim, dtype=torch.float32, device=eng.device)
+            seed, off = eng.latent_stream()
+            z, after = eng.draw_latents(batch, seed, off)
+            eng.set_latent_stream(True, seed, after)
+            return z
         # the sampling step is bit-exact with the oracle: same CPU mt19937 stream, then one H2D copy
         return torch.randn(batch, self.noise_dim, generator=self._latent_gen, dtype=torch.float32)
 
@@ -97,6 +134,8 @@ class ModularGenerator(_CudaModule):
         return eng
 
     def forward(self, h_emb: torch.Tensor, r_emb: torch.Tensor, z: torch.Tensor | None = None) -> torch.Tensor:
+        if z is None and latent_source(self.latent_source) == "cuda":
+            return self._device_stream().generator_forward(h_emb, r_emb, None, precision=self.precision)
         eng = self._get_engine()
         if z is None:
             z = self.sample_latent(h_emb.shape[0])

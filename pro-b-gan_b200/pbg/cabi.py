@@ -24,6 +24,7 @@ SYMBOLS = (
     "pbg_score_triplets_host", "pbg_linear_bf16", "pbg_profile_enable", "pbg_profile_read", "pbg_debug_trace", "pbg_check_indices", "pbg_launch_count",
     "pbg_set_launch_width", "pbg_set_result_mirrors", "pbg_topk_prepare", "pbg_topk", "pbg_parse_index_rows", "pbg_format_f32_json", "pbg_format_i64_json",
     "pbg_reserve", "pbg_stage_triplets", "pbg_score_staged", "pbg_set_result_multicast", "pbg_topk_last_flagged", "pbg_score_triplets_host_packed", "pbg_score_staged_stage_next", "pbg_set_workspace_discard", "pbg_last_pass_sm_clock",
+    "pbg_draw_latents", "pbg_set_latent_stream", "pbg_get_latent_stream", "pbg_score_triplets_host_ids",
 )
 
 
@@ -54,7 +55,7 @@ def load() -> C.CDLL:
     override = os.environ.get("PBG_LIB_PATH")     # an A/B build of the same sources (pbg.build --variant), never a fallback
     path = Path(override) if override else _build.build()
     lib = C.CDLL(str(path))
-    vp, i64, i32, sz = C.c_void_p, C.c_int64, C.c_int, C.c_size_t
+    vp, i64, i32, sz, u64 = C.c_void_p, C.c_int64, C.c_int, C.c_size_t, C.c_uint64
     sig = {
         "pbg_abi_version": (C.c_int, []),
         "pbg_create": (C.c_int, [C.POINTER(vp), C.POINTER(PbgDims)]),
@@ -90,6 +91,10 @@ def load() -> C.CDLL:
         "pbg_topk_last_flagged": (i64, [vp, vp]),
         "pbg_score_triplets_host_packed": (C.c_int, [vp, vp, i64, vp, i64, vp, vp, i64, i32]),
         "pbg_score_staged_stage_next": (C.c_int, [vp, i32, vp, i32, vp, vp, vp, vp, i64, vp, i64, vp, vp, i64, vp]),
+        "pbg_draw_latents": (C.c_int, [vp, u64, u64, i64, i64, i64, vp, C.POINTER(u64), vp]),
+        "pbg_set_latent_stream": (C.c_int, [vp, i32, u64, u64]),
+        "pbg_get_latent_stream": (C.c_int, [vp, C.POINTER(u64), C.POINTER(u64), vp]),
+        "pbg_score_triplets_host_ids": (C.c_int, [vp, vp, i64, vp, i64, vp, vp, i64, i32]),
     }
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)

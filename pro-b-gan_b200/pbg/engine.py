@@ -68,6 +68,7 @@ class Engine:
             self._h = C.c_void_p(0)
             cabi.check(st, None)
         self.g_loaded = self.d_loaded = False
+        self._latent_on = False
         if ctas:
             self.set_launch_width(ctas)
 
@@ -210,11 +211,49 @@ class Engine:
     def launch_count(self) -> int:
         return int(self._lib.pbg_launch_count(self._h))
 
+    # ------------------------------------------------------------------ device latents
+    def set_latent_stream(self, enable: bool = True, seed: int = 0, offset: int = 0) -> None:
+        """Turn the ctx's latent stream on or off (include/pbg.h: pbg_set_latent_stream).  While it is on, every generator
+        call given ``z=None`` draws its [B, Z] latents on the device exactly as ``torch.randn((B, Z), device=...,
+        generator=g)`` would for a CUDA generator at Philox (seed, offset), and advances the offset the same way.
+        Synchronises the device."""
+        with torch.cuda.device(self.device):
+            cabi.check(self._lib.pbg_set_latent_stream(self._h, int(bool(enable)), int(seed), int(offset)), self._h)
+        self._latent_on = bool(enable)
+
+    def latent_stream(self) -> tuple[int, int]:
+        """(seed, offset) of the ctx's latent stream: where the next draw starts.  Synchronises the current stream."""
+        seed, off = C.c_uint64(0), C.c_uint64(0)
+        with torch.cuda.device(self.device):
+            cabi.check(self._lib.pbg_get_latent_stream(self._h, C.byref(seed), C.byref(off), self._stream()), self._h)
+        return int(seed.value), int(off.value)
+
+    def draw_latents(self, rows: int, seed: int, offset: int, row_begin: int = 0,
+                     total_rows: int | None = None) -> tuple[torch.Tensor, int]:
+        """Rows [row_begin, row_begin + rows) of the draw ``torch.randn((total_rows, Z), device=..., generator=g)`` makes
+        for g at Philox (seed, offset) (total_rows defaults to rows), as a new fp32 [rows, Z] tensor; with the offset the
+        generator has after that draw.  Stateless: the ctx's own stream does not move."""
+        total = int(rows if total_rows is None else total_rows)
+        z = torch.empty(int(rows), self.Z, dtype=torch.float32, device=self.device)
+        after = C.c_uint64(0)
+        with torch.cuda.device(self.device):
+            cabi.check(self._lib.pbg_draw_latents(self._h, int(seed), int(offset), total, int(row_begin), int(rows), _ptr(z),
+                                                  C.byref(after), self._stream()), self._h)
+        return z, int(after.value)
+
+    def _latents(self, z, name: str = "z"):
+        """The caller's latents, or None (drawn by the ctx) when the latent stream is on."""
+        if z is not None:
+            return self._f32(z, self.Z, name)
+        if not self._latent_on:
+            raise ValueError("generator pass needs latents z (or the ctx's latent stream: set_latent_stream)")
+        return None
+
     # ------------------------------------------------------------------ generator
-    def generator_forward(self, h, r, z, precision=None, out_dtype=torch.float32) -> torch.Tensor:
-        h, r, z = self._f32(h, self.E, "h_emb"), self._f32(r, self.E, "r_emb"), self._f32(z, self.Z, "z")
+    def generator_forward(self, h, r, z=None, precision=None, out_dtype=torch.float32) -> torch.Tensor:
+        h, r, z = self._f32(h, self.E, "h_emb"), self._f32(r, self.E, "r_emb"), self._latents(z)
         B = h.shape[0]
-        if r.shape[0] != B or z.shape[0] != B:
+        if r.shape[0] != B or (z is not None and z.shape[0] != B):
             raise ValueError("h_emb, r_emb and z must have the same batch size")
         out = torch.empty(B, self.E, dtype=out_dtype, device=self.device)
         with torch.cuda.device(self.device):
@@ -223,12 +262,12 @@ class Engine:
                 cabi.DT_BF16 if out_dtype == torch.bfloat16 else cabi.DT_F32, self._stream()), self._h)
         return out
 
-    def generator_forward_gather(self, node_emb, rel_w, heads, rels, z, precision=None,
+    def generator_forward_gather(self, node_emb, rel_w, heads, rels, z=None, precision=None,
                                  out_dtype=torch.float32) -> torch.Tensor:
         node_emb = self._f32(node_emb, self.E, "node_emb")
         rel_w = self._f32(rel_w, self.E, "rel_emb.weight")
         heads, rels = self._i64(heads, "heads"), self._i64(rels, "relations")
-        z = self._f32(z, self.Z, "z")
+        z = self._latents(z)
         B = heads.shape[0]
         out = torch.empty(B, self.E, dtype=out_dtype, device=self.device)
         with torch.cuda.device(self.device):
@@ -284,9 +323,7 @@ class Engine:
         B = trip.shape[0]
         run_g = want_gen_out or want_gen_scores
         if run_g:
-            if z is None:
-                raise ValueError("generator pass needs latents z")
-            z = self._f32(z, self.Z, "z")
+            z = self._latents(z)
         res = {}
         out = out or {}
 
@@ -335,9 +372,7 @@ class Engine:
             raise ValueError(f"triplets must be [B, 3], got {tuple(trip.shape)}")
         trip = trip.contiguous()
         if want_gen:
-            if z is None:
-                raise ValueError("generator pass needs latents z")
-            z = self._f32(z, self.Z, "z")
+            z = self._latents(z)
         B = trip.shape[0]
         with torch.cuda.device(self.device):
             cabi.check(self._lib.pbg_stage_triplets(
@@ -387,9 +422,7 @@ class Engine:
                     raise ValueError("the next request's triplets must be a contiguous [B, 3] tensor")
                 run_g = want_gen_out or want_gen_scores
                 if run_g:
-                    if n_z is None:
-                        raise ValueError("generator pass needs latents z")
-                    n_z = self._f32(n_z, self.Z, "z")
+                    n_z = self._latents(n_z)
                 cabi.check(self._lib.pbg_score_staged_stage_next(
                     self._h, int(slot), _ptr(gen_out), dt, _ptr(scores), _ptr(logits), _ptr(probs), _ptr(n_emb), n_emb.shape[0],
                     _ptr(n_rel), n_rel.shape[0], _ptr(n_trip), _ptr(n_z if run_g else None), n_trip.shape[0], self._stream()),
@@ -437,4 +470,24 @@ class Engine:
         with torch.cuda.device(self.device):
             cabi.check(self._lib.pbg_score_triplets_host_packed(
                 self._h, _ptr(node_emb), node_emb.shape[0], _ptr(rel_w), rel_w.shape[0], _ptr(in_block_host),
+                _ptr(out_block_host), B, precision_code(precision)), self._h)
+
+    def score_triplets_host_ids(self, node_emb, rel_w, triplets_host: torch.Tensor, out_block_host: torch.Tensor,
+                                precision=None) -> None:
+        """pbg_score_triplets_host_ids: only the ids travel -- ``triplets_host`` int64 [B, 3] in, ``out_block_host`` fp32
+        [3 B] = [gen_scores | logits | probs] out -- and the latents come from the ctx's latent stream, which must be on.
+        One copy per direction, one sync."""
+        if triplets_host.device.type != "cpu" or out_block_host.device.type != "cpu":
+            raise ValueError("the blocks must be CPU (ideally pinned) tensors")
+        if triplets_host.dtype != torch.int64 or triplets_host.dim() != 2 or triplets_host.shape[1] != 3 \
+                or not triplets_host.is_contiguous():
+            raise ValueError("triplets_host must be a contiguous int64 [B, 3] tensor")
+        B = triplets_host.shape[0]
+        if out_block_host.dtype != torch.float32 or out_block_host.numel() != 3 * B or not out_block_host.is_contiguous():
+            raise ValueError(f"out_block_host must be a contiguous fp32 tensor of {3 * B} elements")
+        if not self._latent_on:
+            raise ValueError("score_triplets_host_ids draws the latents on the device: call set_latent_stream first")
+        with torch.cuda.device(self.device):
+            cabi.check(self._lib.pbg_score_triplets_host_ids(
+                self._h, _ptr(node_emb), node_emb.shape[0], _ptr(rel_w), rel_w.shape[0], _ptr(triplets_host),
                 _ptr(out_block_host), B, precision_code(precision)), self._h)

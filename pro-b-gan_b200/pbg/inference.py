@@ -29,7 +29,11 @@ from .analyze import analyze_relations_batched
 
 
 class FusedInference:
-    def __init__(self, checkpoint_path: str, device: str = "auto", precision: str | None = None, verbose: bool = False):
+    def __init__(self, checkpoint_path: str, device: str = "auto", precision: str | None = None, verbose: bool = False,
+                 latents: str | None = None):
+        """``latents``: 'cpu' (default; PBG_LATENTS overrides) draws z from the generator's CPU mt19937 stream, as the
+        oracle does, and ships it with the ids; 'cuda' draws z on the device from a Philox stream seeded LATENT_SEED
+        (what torch.randn(..., device='cuda', generator=g) gives), so only ids cross PCIe."""
         import modular_prot_b_gan as m
         if device in ("auto", "cuda"):
             if not torch.cuda.is_available():
@@ -64,6 +68,9 @@ class FusedInference:
         self.generator.precision = self.discriminator.precision = precision
         t2 = time.perf_counter()
         self.engine = m.make_fused_engine(self.generator, self.discriminator)       # BN fold + bf16 pack + upload
+        self.latents = m.latent_source(latents)
+        if self.latents == "cuda":
+            self.engine.set_latent_stream(True, m.LATENT_SEED, 0)
         torch.cuda.synchronize(self.device)
         t3 = time.perf_counter()
         self.best_val_hit10 = ckpt.get("best_val_hit10", 0.0)
@@ -75,6 +82,14 @@ class FusedInference:
         if verbose:
             print(f"FusedInference ready: {self.num_entities:,} entities, {self.num_relations:,} relations, "
                   f"E={self.embed_dim}; ingest {self.ingest_ms}")
+
+    def reseed(self, seed: int | None = None) -> None:
+        """Restart the latent stream this object draws from (CPU generator or device stream) at `seed`."""
+        import modular_prot_b_gan as m
+        seed = m.LATENT_SEED if seed is None else int(seed)
+        self.generator.reseed(seed)
+        if self.latents == "cuda":
+            self.engine.set_latent_stream(True, seed, 0)
 
     # ------------------------------------------------------------------ helpers
     def _pin(self, name: str, rows: int, shape_tail: tuple, dtype) -> torch.Tensor:
@@ -122,13 +137,20 @@ class FusedInference:
         run_g, run_d = method in ("generator", "both"), method in ("discriminator", "both")
         if not (run_g or run_d):
             return results                                   # an unknown method yields metadata only, as :196-209
-        z = self._latents(B) if run_g else None
-        scores = self._pin("gen_scores", B, (), torch.float32) if run_g else None
-        logits = self._pin("logits", B, (), torch.float32) if run_d else None
-        probs = self._pin("probs", B, (), torch.float32) if run_d else None
-        with torch.cuda.device(self.device):
-            self.engine.score_triplets_host(self.node_emb, self.rel_weight, trip, z, None, scores, logits, probs,
-                                            precision=self.precision)   # raises IndexError on a bad id
+        if self.latents == "cuda" and run_g and run_d:
+            # only the ids travel: [triplets] in, [gen_scores | logits | probs] out, latents drawn on the device
+            block = self._pin("out_block", 3 * B, (), torch.float32)
+            scores, logits, probs = block[:B], block[B:2 * B], block[2 * B:]
+            with torch.cuda.device(self.device):
+                self.engine.score_triplets_host_ids(self.node_emb, self.rel_weight, trip, block, precision=self.precision)
+        else:
+            z = self._latents(B) if run_g and self.latents == "cpu" else None
+            scores = self._pin("gen_scores", B, (), torch.float32) if run_g else None
+            logits = self._pin("logits", B, (), torch.float32) if run_d else None
+            probs = self._pin("probs", B, (), torch.float32) if run_d else None
+            with torch.cuda.device(self.device):
+                self.engine.score_triplets_host(self.node_emb, self.rel_weight, trip, z, None, scores, logits, probs,
+                                                precision=self.precision)   # raises IndexError on a bad id
         if run_g:
             results["generator_scores"] = out(scores)
         if run_d:
@@ -146,7 +168,7 @@ class FusedInference:
         with torch.no_grad(), torch.cuda.device(self.device):
             try:
                 dev_pairs = pairs.to(self.device, non_blocking=True)
-                z = self._latents(B).to(self.device, non_blocking=True)
+                z = self._latents(B).to(self.device, non_blocking=True) if self.latents == "cpu" else None
                 pred = self.engine.generator_forward_gather(self.node_emb, self.rel_weight, dev_pairs[:, 0], dev_pairs[:, 1],
                                                             z, precision=self.precision)
                 top_scores, top_idx = self.engine.cosine_topk(pred, self.node_emb, top_k)
