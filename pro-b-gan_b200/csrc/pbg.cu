@@ -50,12 +50,10 @@ inline int round_up(int v, int m) { return (v + m - 1) / m * m; }
 struct Linear {
   int n = 0, k = 0;    // logical [out, in]
   int np = 0, kp = 0;  // padded to the tensor-core tile grid
-  int block_n = 0;
   float* w_f32 = nullptr;
   float* b_f32 = nullptr;
   __nv_bfloat16* w_bf16 = nullptr;
   float* b_pad = nullptr;
-  CUtensorMap tmap_w;     // box 64 x block_n
   CUtensorMap tmap_w128;  // box 64 x 128 (finer tiles for small batches; one CTA's half of a 256-wide pair tile)
   CUtensorMap tmap_w64;   // box 64 x 64  (one CTA's half of a 128-wide pair tile)
 };
@@ -113,7 +111,7 @@ struct pbg_ctx {
   int num_sms = 0;
   int max_threads_sm = 0;   // with num_sms, sets torch's launch geometry that the latent draw reproduces
   bool g_loaded = false, d_loaded = false;
-  int kg0 = 0, kg0p = 0, kd0 = 0, kd0p = 0, hgp = 0, hdp = 0, hd2 = 0, hd2p = 0, ep = 0, hmax = 0;
+  int kg0 = 0, kg0p = 0, kd0 = 0, kd0p = 0, hgp = 0, hdp = 0, hd2 = 0, hmax = 0;
   Linear g[3], d[2];
   float* d_w3 = nullptr;      // [hd2] fp32
   float* d_w3_pad = nullptr;  // [hd2p]
@@ -127,8 +125,6 @@ struct pbg_ctx {
   // host buffers the caller laid out the same way travel in one copy per direction
   long long host_cap = 0;
   char* st_block = nullptr;
-  long long* st_trip = nullptr;
-  float *st_z = nullptr, *st_gen = nullptr, *st_scores = nullptr, *st_logits = nullptr, *st_probs = nullptr;
   EncodeTiledFn encode = nullptr;
   TopkState tk;
   // latent stream (pbg_set_latent_stream): generator calls without z draw from Philox (lat_seed, lat_st->offset)
@@ -215,12 +211,11 @@ void free_ws(Workspace& w) {
   w = Workspace{};
 }
 
-// Upload one Linear: fp32 copy for the parity mode, padded bf16 copy + TMA descriptor for the tensor-core mode.
+// Upload one Linear: fp32 copy for the parity mode, padded bf16 copy + TMA descriptors for the tensor-core mode.
 int upload_linear(pbg_ctx* c, Linear& l, int n, int k, int kp, const float* w_host, const float* b_host) {
   free_linear(l);
   l.n = n; l.k = k; l.kp = kp;
   l.np = round_up(n, 128);
-  l.block_n = (l.np % 256 == 0) ? 256 : 128;
   PBG_CUDA(c, cudaMalloc(&l.w_f32, sizeof(float) * n * k));
   PBG_CUDA(c, cudaMalloc(&l.b_f32, sizeof(float) * n));
   PBG_CUDA(c, cudaMalloc(&l.w_bf16, sizeof(__nv_bfloat16) * (size_t)l.np * l.kp));
@@ -234,17 +229,33 @@ int upload_linear(pbg_ctx* c, Linear& l, int n, int k, int kp, const float* w_ho
   PBG_CUDA(c, cudaGetLastError());
   PBG_CUDA(c, cudaStreamSynchronize(c->own_stream));
   PBG_TRY(make_tmap(c, &l.tmap_w128, l.w_bf16, l.np, l.kp, 128));
-  PBG_TRY(make_tmap(c, &l.tmap_w64, l.w_bf16, l.np, l.kp, 64));
-  return make_tmap(c, &l.tmap_w, l.w_bf16, l.np, l.kp, l.block_n);
+  return make_tmap(c, &l.tmap_w64, l.w_bf16, l.np, l.kp, 64);
 }
 
 // Growing a buffer means cudaDeviceSynchronize + cudaFree + cudaMalloc: illegal while `s` is being captured into a
 // CUDA graph, and a device-wide stall for every other lane otherwise -- callers that care size everything up front
-// with pbg_reserve().
-int refuse_growth_in_capture(pbg_ctx* c, cudaStream_t s, const char* what) {
+// with pbg_reserve().  Refuses inside a capture, otherwise waits until nothing may still be reading the old buffers.
+int begin_growth(pbg_ctx* c, cudaStream_t s, const char* what) {
   cudaStreamCaptureStatus st = cudaStreamCaptureStatusNone;
   if (cudaStreamIsCapturing(s, &st) == cudaSuccess && st != cudaStreamCaptureStatusNone)
     return fail(c, PBG_ERR_INVALID, "%s must grow while the stream is being captured: call pbg_reserve() first", what);
+  PBG_CUDA(c, cudaDeviceSynchronize());
+  return PBG_OK;
+}
+
+// Rows to allocate for `rows`: rounded up to a power of two in [1024, kMaxChunk], so that small calls do not keep
+// reallocating.
+long long pow2_cap(long long rows) {
+  long long cap = 1024;
+  while (cap < rows) cap *= 2;
+  return std::min(cap, kMaxChunk);
+}
+
+// Replaces *p by a fresh allocation of `bytes`; *p is null if that fails.
+template <class T>
+int realloc_dev(pbg_ctx* c, T*& p, size_t bytes) {
+  cudaFree(p); p = nullptr;
+  PBG_CUDA(c, cudaMalloc(&p, bytes));
   return PBG_OK;
 }
 
@@ -256,12 +267,8 @@ void free_stage(StageSlot& st) {
 int ensure_ws(pbg_ctx* c, int prec, long long rows, cudaStream_t stream) {
   Workspace& w = prec == PBG_PREC_BF16 ? c->ws_bf16 : c->ws_f32;
   if (w.rows >= rows) return PBG_OK;
-  PBG_TRY(refuse_growth_in_capture(c, stream, "the workspace"));
-  // round the capacity up so that small calls do not keep reallocating
-  long long cap = 1024;
-  while (cap < rows) cap *= 2;
-  cap = std::min(cap, kMaxChunk);
-  PBG_CUDA(c, cudaDeviceSynchronize());  // nothing may still be reading the old buffers
+  PBG_TRY(begin_growth(c, stream, "the workspace"));
+  const long long cap = pow2_cap(rows);
   free_ws(w);
   if (prec == PBG_PREC_BF16) {
     const size_t es = sizeof(__nv_bfloat16);
@@ -302,11 +309,8 @@ int ensure_ws(pbg_ctx* c, int prec, long long rows, cudaStream_t stream) {
 
 int ensure_stage(pbg_ctx* c, StageSlot& st, long long rows, cudaStream_t stream) {
   if (st.cap >= rows) return PBG_OK;
-  PBG_TRY(refuse_growth_in_capture(c, stream, "a staging slot"));
-  long long cap = 1024;
-  while (cap < rows) cap *= 2;
-  cap = std::min(cap, kMaxChunk);
-  PBG_CUDA(c, cudaDeviceSynchronize());  // nothing may still be reading the old buffers
+  PBG_TRY(begin_growth(c, stream, "a staging slot"));
+  const long long cap = pow2_cap(rows);
   free_stage(st);
   const size_t es = sizeof(__nv_bfloat16);
   PBG_CUDA(c, cudaMalloc(&st.xg0, es * cap * c->kg0p));
@@ -321,13 +325,10 @@ int ensure_stage(pbg_ctx* c, StageSlot& st, long long rows, cudaStream_t stream)
 
 int ensure_latents(pbg_ctx* c, long long rows, cudaStream_t stream) {
   if (c->lat_cap >= rows) return PBG_OK;
-  PBG_TRY(refuse_growth_in_capture(c, stream, "the latent workspace"));
-  long long cap = 1024;
-  while (cap < rows) cap *= 2;
-  cap = std::min(cap, kMaxChunk);
-  PBG_CUDA(c, cudaDeviceSynchronize());  // nothing may still be reading the old buffer
-  cudaFree(c->lat_z); c->lat_z = nullptr; c->lat_cap = 0;
-  PBG_CUDA(c, cudaMalloc(&c->lat_z, sizeof(float) * cap * c->dims.noise_dim));
+  PBG_TRY(begin_growth(c, stream, "the latent workspace"));
+  const long long cap = pow2_cap(rows);
+  c->lat_cap = 0;
+  PBG_TRY(realloc_dev(c, c->lat_z, sizeof(float) * cap * c->dims.noise_dim));
   c->lat_cap = cap;
   return PBG_OK;
 }
@@ -423,7 +424,7 @@ int run_chunk(pbg_ctx* c, const Pass& a, long long off, long long rows) {
   gp.xd = a.run_d ? w.xd0 : nullptr; gp.ldd = bf ? c->kd0p : c->kd0;
   gp.B = rows; gp.err_flag = c->err_flag;
   const int gather_blocks = (int)std::min<long long>((rows + 7) / 8, (long long)c->num_sms * 8);
-  if (!bf && (c->n_mirror > 0 || c->mc_gen || c->mc_cos || c->mc_logits))
+  if (!bf && (c->n_mirror > 0 || c->mc_gen || c->mc_cos || c->mc_logits || c->mc_probs))
     return fail(c, PBG_ERR_UNSUPPORTED, "result mirrors / multicast are a bf16-mode feature");
   // bf16 mode gathers inside the fused pass kernel.  PBG_SPLIT_GATHER=1 (experiment, see DESIGN.md 3.1 "time model"):
   // the rows are gathered by this small kernel instead -- it fits beside resident pass CTAs of other lanes (no shared
@@ -475,22 +476,46 @@ int run_chunk(pbg_ctx* c, const Pass& a, long long off, long long rows) {
 }
 
 
-template <bool TR, bool FASTG, bool BIASS>
-cudaError_t launch_p2(pbg_ctx* c, const Pass2Params& p, int grid, cudaStream_t s, bool pdl) {
-  auto kern = pbg_pass2_kernel<TR, FASTG, BIASS>;
-  static int attr_dev = -1;  // per instantiation; ctxs on different devices share the function handle
-  if (attr_dev != c->dims.device) {
-    const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, P2Smem::kTotal);
-    if (e != cudaSuccess) return e;
-    attr_dev = c->dims.device;
-  }
+// launch with programmatic stream serialisation (pdl): the kernel may begin while its predecessor on the stream drains; it
+// orders itself behind the predecessor with griddepcontrol.wait (topk_kernel.cuh: pdl_wait).  Used for the pass kernel
+// (PBG_PDL) and, in top-k, for the kernels of one CTA per SM (sample, scan: their prologue -- barriers, TMEM,
+// descriptors -- overlaps the predecessor's tail) and for the exact-scan launch.  NOT for the cut-off and rescoring kernels: their many small blocks, released early, pile onto
+// whichever SMs the cluster kernel before them left idle (20 of 148 behind the sample launch, 34 behind a 1024-row scan)
+// instead of spreading over the device -- measured per link at k = 64: cut-off +12 / +32 us at B = 1024 / 4096, rescore
+// +33 us at B = 1024; sample, scan, exact: -3 us each (B = 256, k = 10: 84.5 -> 76 us).
+template <class... KArgs, class... Args>
+cudaError_t launch_pdl(bool pdl, void (*kern)(KArgs...), unsigned grid, unsigned block, size_t smem, cudaStream_t s, Args&&... args) {
   cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(grid); cfg.blockDim = dim3(kP2Threads); cfg.dynamicSmemBytes = P2Smem::kTotal; cfg.stream = s;
+  cfg.gridDim = dim3(grid); cfg.blockDim = dim3(block); cfg.dynamicSmemBytes = smem; cfg.stream = s;
   cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   at[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = at; cfg.numAttrs = pdl ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kern, p);
+  return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
+}
+
+// The pass kernel's instantiations, indexed by (TR ? 4 : 0) | (FASTG ? 2 : 0) | (BIASS ? 1 : 0).
+using Pass2Kernel = void (*)(Pass2Params);
+const Pass2Kernel kPass2[8] = {
+    pbg_pass2_kernel<false, false, false>, pbg_pass2_kernel<false, false, true>, pbg_pass2_kernel<false, true, false>,
+    pbg_pass2_kernel<false, true, true>,   pbg_pass2_kernel<true, false, false>, pbg_pass2_kernel<true, false, true>,
+    pbg_pass2_kernel<true, true, false>,   pbg_pass2_kernel<true, true, true>};
+
+// Per layer kind (IT_*): its epilogue, the counter that gates its A operand, the counter its stores bump.
+const int kEpiOf[5] = {PEPI_STORE, PEPI_STORE, PEPI_STORE, PEPI_ROWDOT, PEPI_TANH};
+const int kPredOf[5] = {DEP_X, DEP_X, DEP_G0, DEP_D0, DEP_G1};
+const int kOutOf[5] = {DEP_G0, DEP_D0, DEP_G1, -1, -1};
+
+// Layer kind k of a pass over Linear l: its A operand `amap`, the store map `omap` and rows `out` (leading dimension
+// `ldo`) of a PEPI_STORE layer.  Tiles are 256 x 256, or 256 x 128 when the padded width is not a multiple of 256.
+void set_layer(Pass2Params& p, int k, const Linear& l, const CUtensorMap& amap, const CUtensorMap* omap,
+               __nv_bfloat16* out, int ldo) {
+  const int bn = (l.np % 256 == 0) ? 256 : 128;
+  p.tm_a[k] = amap;
+  p.tm_w[k] = bn == 256 ? l.tmap_w128 : l.tmap_w64;
+  if (omap) p.tm_o[k] = *omap;
+  p.layer[k] = P2Layer{l.kp / kBlockK, bn, l.np / bn, kEpiOf[k], kPredOf[k], kOutOf[k], ldo, -1, l.b_pad, out};
+  p.layer_mask |= 1u << k;
 }
 
 // The pair kernel (pass2_kernel.cuh): 256-row blocks, tiles of 256 x {256 | 128}, one CTA pair per tile.
@@ -505,24 +530,15 @@ int launch_pass2(pbg_ctx* c, Workspace& w, const Pass& a, const GatherParams& gp
                                 &w.tm_bufB_g};
   const CUtensorMap* omap[5] = {&w.tmo_bufA, &w.tmo_bufD, &w.tmo_bufB, nullptr, nullptr};
   const bool on[5] = {a.run_g, a.run_d, a.run_g, a.run_d, a.run_g};
-  static const int pred_of[5] = {DEP_X, DEP_X, DEP_G0, DEP_D0, DEP_G1};
-  static const int out_of[5] = {DEP_G0, DEP_D0, DEP_G1, -1, -1};
-  static const int epi_of[5] = {PEPI_STORE, PEPI_STORE, PEPI_STORE, PEPI_ROWDOT, PEPI_TANH};
   const int nrb = static_cast<int>((rows + kP2Rows - 1) / kP2Rows);
   __nv_bfloat16* outs[5] = {(__nv_bfloat16*)w.bufA, (__nv_bfloat16*)w.bufD, (__nv_bfloat16*)w.bufB, nullptr, nullptr};
   const int ldos[5] = {c->hgp, c->hdp, c->hgp, 0, 0};
   long long total = 0;
   for (int k = 0; k < 5; ++k) {
     if (!on[k]) continue;
-    const Linear& l = *lin[k];
-    const int bn = (l.np % 256 == 0) ? 256 : 128;
-    if (l.np / bn > 255) return fail(c, PBG_ERR_UNSUPPORTED, "layer too wide for the tile index");
-    p.tm_a[k] = *amap[k];
-    p.tm_w[k] = bn == 256 ? l.tmap_w128 : l.tmap_w64;
-    if (omap[k]) p.tm_o[k] = *omap[k];
-    p.layer[k] = P2Layer{l.kp / kBlockK, bn, l.np / bn, epi_of[k], pred_of[k], out_of[k], ldos[k], -1, l.b_pad, outs[k]};
-    p.layer_mask |= 1u << k;
-    total += static_cast<long long>(nrb) * (l.np / bn);
+    set_layer(p, k, *lin[k], *amap[k], omap[k], outs[k], ldos[k]);
+    if (p.layer[k].n_tiles > 255) return fail(c, PBG_ERR_UNSUPPORTED, "layer too wide for the tile index");
+    total += static_cast<long long>(nrb) * p.layer[k].n_tiles;
   }
   // biases + final dot weights are copied to shared memory at kernel start when they fit (H <= 1024)
   bool biass = false;
@@ -634,23 +650,14 @@ int launch_pass2(pbg_ctx* c, Workspace& w, const Pass& a, const GatherParams& gp
   static const bool pdl = [] { const char* e = getenv("PBG_PDL"); return !e || atoi(e) != 0; }();
   const bool fastg = c->dims.embed_dim == 128 && c->dims.noise_dim % 4 == 0 && c->dims.noise_dim <= 128 &&
                      c->kg0p == c->kg0 && c->kd0p == c->kd0;  // the bulk-store gather writes unpadded rows
+  const Pass2Kernel kern = kPass2[(p.trace ? 4 : 0) | (fastg ? 2 : 0) | (biass ? 1 : 0)];
   cudaError_t le;
   { LaunchScope ls(c, PBG_K_PASS, a.stream);
-    const int sel = (p.trace ? 4 : 0) | (fastg ? 2 : 0) | (biass ? 1 : 0);
-    switch (sel) {
-      case 0: le = launch_p2<false, false, false>(c, p, grid, a.stream, pdl); break;
-      case 1: le = launch_p2<false, false, true>(c, p, grid, a.stream, pdl); break;
-      case 2: le = launch_p2<false, true, false>(c, p, grid, a.stream, pdl); break;
-      case 3: le = launch_p2<false, true, true>(c, p, grid, a.stream, pdl); break;
-      case 4: le = launch_p2<true, false, false>(c, p, grid, a.stream, pdl); break;
-      case 5: le = launch_p2<true, false, true>(c, p, grid, a.stream, pdl); break;
-      case 6: le = launch_p2<true, true, false>(c, p, grid, a.stream, pdl); break;
-      default: le = launch_p2<true, true, true>(c, p, grid, a.stream, pdl); break;
-    } }
+    le = launch_pdl(pdl, kern, grid, kP2Threads, P2Smem::kTotal, a.stream, p); }
   if (le == cudaSuccess) le = cudaGetLastError();
   if (le != cudaSuccess) {
     cudaFuncAttributes fa{};
-    cudaFuncGetAttributes(&fa, pbg_pass2_kernel<false, true, true>);
+    cudaFuncGetAttributes(&fa, kern);
     return fail(c, PBG_ERR_CUDA, "pass kernel launch failed: %s (grid %d x %d threads, %d regs/thread, %zu B static + %d B dynamic smem, "
                 "max threads/block %d, max dynamic smem %d)", cudaGetErrorString(le), grid, kP2Threads, fa.numRegs,
                 fa.sharedSizeBytes, P2Smem::kTotal, fa.maxThreadsPerBlock, fa.maxDynamicSharedSizeBytes);
@@ -679,26 +686,6 @@ int run_pass(pbg_ctx* c, Pass a) {
   return PBG_OK;
 }
 
-}  // namespace
-
-namespace {
-// launch with programmatic stream serialisation (pdl): the kernel may begin while its predecessor on the stream drains; it
-// orders itself behind the predecessor with griddepcontrol.wait (topk_kernel.cuh: pdl_wait).  Used for the kernels of
-// one CTA per SM (sample, scan: their prologue -- barriers, TMEM, descriptors -- overlaps the predecessor's tail) and for
-// the exact-scan launch.  NOT for the cut-off and rescoring kernels: their many small blocks, released early, pile onto
-// whichever SMs the cluster kernel before them left idle (20 of 148 behind the sample launch, 34 behind a 1024-row scan)
-// instead of spreading over the device -- measured per link at k = 64: cut-off +12 / +32 us at B = 1024 / 4096, rescore
-// +33 us at B = 1024; sample, scan, exact: -3 us each (B = 256, k = 10: 84.5 -> 76 us).
-template <class... KArgs, class... Args>
-cudaError_t launch_pdl(bool pdl, void (*kern)(KArgs...), unsigned grid, unsigned block, size_t smem, cudaStream_t s, Args&&... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(grid); cfg.blockDim = dim3(block); cfg.dynamicSmemBytes = smem; cfg.stream = s;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  at[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = at; cfg.numAttrs = pdl ? 1 : 0;
-  return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
-}
 }  // namespace
 
 extern "C" {
@@ -738,10 +725,10 @@ int pbg_topk_prepare(pbg_ctx* c, const float* table, int64_t N, void* stream) {
   TopkState& t = c->tk;
   const long long n_pad = (N + 255) / 256 * 256;
   if (n_pad != t.n_pad) {
-    PBG_CUDA(c, cudaDeviceSynchronize());
-    cudaFree(t.tn); cudaFree(t.inv_t); t.tn = nullptr; t.inv_t = nullptr; t.n_pad = 0;
-    PBG_CUDA(c, cudaMalloc(&t.tn, sizeof(__nv_bfloat16) * n_pad * E));
-    PBG_CUDA(c, cudaMalloc(&t.inv_t, sizeof(float) * n_pad));
+    PBG_TRY(begin_growth(c, s, "the top-k table"));
+    t.n_pad = 0;
+    PBG_TRY(realloc_dev(c, t.tn, sizeof(__nv_bfloat16) * n_pad * E));
+    PBG_TRY(realloc_dev(c, t.inv_t, sizeof(float) * n_pad));
     t.n_pad = n_pad;
     if (E == 128) PBG_TRY(make_tmap(c, &t.tm_t, t.tn, n_pad, E, 128));
   }
@@ -764,19 +751,13 @@ int topk_general(pbg_ctx* c, TopkState& t, const float* q, long long rows, int k
   const long long chunk = std::max<long long>(64, std::min<long long>(rows, (512ll << 20) / (4 * t.N)));
   const size_t need = static_cast<size_t>(chunk) * t.N;
   if (t.score_cap < need) {
-    PBG_TRY(refuse_growth_in_capture(c, s, "the top-k score buffer"));
-    PBG_CUDA(c, cudaDeviceSynchronize());
-    cudaFree(t.score_buf); t.score_buf = nullptr; t.score_cap = 0;
-    PBG_CUDA(c, cudaMalloc(&t.score_buf, sizeof(float) * need));
+    PBG_TRY(begin_growth(c, s, "the top-k score buffer"));
+    t.score_cap = 0;
+    PBG_TRY(realloc_dev(c, t.score_buf, sizeof(float) * need));
     t.score_cap = need;
   }
   const int threads = std::max(32, std::min(256, (200 * 1024 / (k * 8)) / 32 * 32));
   const size_t smem = static_cast<size_t>(E) * 4 + static_cast<size_t>(threads) * k * 8;
-  static int attr_dev = -1;
-  if (attr_dev != c->dims.device) {
-    PBG_CUDA(c, cudaFuncSetAttribute(topk_exact_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
-    attr_dev = c->dims.device;
-  }
   for (long long off = 0; off < rows; off += chunk) {
     const long long r = std::min(chunk, rows - off);
     F32GemmParams gp{q + off * E, E, t.table, E, nullptr, t.score_buf, t.N, (int)r, (int)t.N, E, 0.f};
@@ -828,14 +809,12 @@ int pbg_topk(pbg_ctx* c, const float* queries, int64_t B, int k, int64_t* out_id
     const long long rows_pad = (rows + 255) / 256 * 256;
     const float* q = queries + off * E;
     if (t.q_cap < rows_pad) {
-      PBG_TRY(refuse_growth_in_capture(c, s, "the top-k query buffers"));
-      PBG_CUDA(c, cudaDeviceSynchronize());
-      cudaFree(t.qn); cudaFree(t.inv_q); cudaFree(t.flag); cudaFree(t.tau);
-      t.qn = nullptr; t.inv_q = nullptr; t.flag = nullptr; t.tau = nullptr; t.q_cap = 0;
-      PBG_CUDA(c, cudaMalloc(&t.qn, sizeof(__nv_bfloat16) * rows_pad * E));
-      PBG_CUDA(c, cudaMalloc(&t.inv_q, sizeof(float) * rows_pad));
-      PBG_CUDA(c, cudaMalloc(&t.flag, sizeof(int) * rows_pad));
-      PBG_CUDA(c, cudaMalloc(&t.tau, sizeof(float) * rows_pad));
+      PBG_TRY(begin_growth(c, s, "the top-k query buffers"));
+      t.q_cap = 0;
+      PBG_TRY(realloc_dev(c, t.qn, sizeof(__nv_bfloat16) * rows_pad * E));
+      PBG_TRY(realloc_dev(c, t.inv_q, sizeof(float) * rows_pad));
+      PBG_TRY(realloc_dev(c, t.flag, sizeof(int) * rows_pad));
+      PBG_TRY(realloc_dev(c, t.tau, sizeof(float) * rows_pad));
       t.q_cap = rows_pad;
       if (E == 128) PBG_TRY(make_tmap(c, &t.tm_q, t.qn, rows_pad, E, 128));
     }
@@ -882,25 +861,16 @@ int pbg_topk(pbg_ctx* c, const float* queries, int64_t B, int k, int64_t* out_id
     const size_t need = static_cast<size_t>(rows_pad) * n_lists * kTkCand;
     const size_t sneed = static_cast<size_t>(rows_pad) * n_slists * kTkKeys;
     if (t.cand_cap < need || t.samp_cap < sneed) {
-      PBG_TRY(refuse_growth_in_capture(c, s, "the top-k candidate buffers"));
-      PBG_CUDA(c, cudaDeviceSynchronize());
-      cudaFree(t.cand_grp); cudaFree(t.cand_mask); cudaFree(t.cand_cnt); cudaFree(t.samp_keys);
-      t.cand_grp = t.cand_mask = nullptr; t.cand_cnt = nullptr; t.samp_keys = nullptr; t.cand_cap = t.samp_cap = 0;
-      PBG_CUDA(c, cudaMalloc(&t.cand_grp, sizeof(unsigned) * need));
-      PBG_CUDA(c, cudaMalloc(&t.cand_mask, sizeof(unsigned) * need));
-      PBG_CUDA(c, cudaMalloc(&t.cand_cnt, sizeof(int) * need / kTkCand));
-      PBG_CUDA(c, cudaMalloc(&t.samp_keys, sizeof(int) * sneed));
+      PBG_TRY(begin_growth(c, s, "the top-k candidate buffers"));
+      t.cand_cap = t.samp_cap = 0;
+      PBG_TRY(realloc_dev(c, t.cand_grp, sizeof(unsigned) * need));
+      PBG_TRY(realloc_dev(c, t.cand_mask, sizeof(unsigned) * need));
+      PBG_TRY(realloc_dev(c, t.cand_cnt, sizeof(int) * need / kTkCand));
+      PBG_TRY(realloc_dev(c, t.samp_keys, sizeof(int) * sneed));
       t.cand_cap = need; t.samp_cap = sneed;
     }
     ps.samp_keys = t.samp_keys;
     pm.tau = t.tau; pm.cand_grp = t.cand_grp; pm.cand_mask = t.cand_mask; pm.cand_cnt = t.cand_cnt;
-    static int attr_dev = -1;
-    if (attr_dev != c->dims.device) {
-      PBG_CUDA(c, cudaFuncSetAttribute(pbg_topk_scan_kernel<TK_SAMPLE>, cudaFuncAttributeMaxDynamicSharedMemorySize, TkSmem::kTotal));
-      PBG_CUDA(c, cudaFuncSetAttribute(pbg_topk_scan_kernel<TK_SCAN>, cudaFuncAttributeMaxDynamicSharedMemorySize, TkSmem::kTotal));
-      PBG_CUDA(c, cudaFuncSetAttribute(topk_exact_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024));
-      attr_dev = c->dims.device;
-    }
     { LaunchScope ls(c, PBG_K_TOPK, s);
       PBG_CUDA(c, launch_pdl(true, pbg_topk_scan_kernel<TK_SAMPLE>, std::min(grid, 2 * ((ps.total + ps.span - 1) / ps.span)), kPassThreads, TkSmem::kTotal, s, ps)); }
     { LaunchScope ls(c, PBG_K_OTHER, s);
@@ -1013,11 +983,18 @@ int pbg_create(pbg_ctx** out, const pbg_dims* dims) {
   c->kg0 = 2 * E + Z; c->kg0p = round_up(c->kg0, kBlockK);
   c->kd0 = 3 * E;     c->kd0p = round_up(c->kd0, kBlockK);
   c->hgp = round_up(HG, 128); c->hdp = round_up(HD, 128);
-  c->hd2 = HD / 2; c->hd2p = round_up(c->hd2, 128);
-  c->ep = round_up(E, 128);
+  c->hd2 = HD / 2;
   c->hmax = std::max(c->hgp, c->hdp);
   auto bail = [&](int code) { g_create_error = c->err; pbg_destroy(c); return code; };
   if (cudaSetDevice(dims->device) != cudaSuccess) { c->err = "cudaSetDevice failed"; return bail(PBG_ERR_CUDA); }
+  // the dynamic shared memory of the kernels that take more than the default 48 KB, on this ctx's device
+  e = cudaSuccess;
+  for (Pass2Kernel k : kPass2)
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, P2Smem::kTotal);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(pbg_topk_scan_kernel<TK_SAMPLE>, cudaFuncAttributeMaxDynamicSharedMemorySize, TkSmem::kTotal);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(pbg_topk_scan_kernel<TK_SCAN>, cudaFuncAttributeMaxDynamicSharedMemorySize, TkSmem::kTotal);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(topk_exact_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 220 * 1024);
+  if (e != cudaSuccess) { c->err = std::string("cudaFuncSetAttribute failed: ") + cudaGetErrorString(e); return bail(PBG_ERR_CUDA); }
   void* fn = nullptr;
   cudaDriverEntryPointQueryResult qres;
   if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &fn, cudaEnableDefault, &qres) != cudaSuccess || !fn) {
@@ -1208,6 +1185,36 @@ int pbg_get_latent_stream(pbg_ctx* c, uint64_t* seed, uint64_t* offset, void* st
   return PBG_OK;
 }
 
+namespace {
+// The gather of a [B, 3] triplet request into staging slot `st`: the generator's first-layer rows (when `gen`) and the
+// discriminator's (when `disc`).
+GatherParams slot_gather(const pbg_ctx* c, const StageSlot& st, const float* node_emb, long long N, const float* rel_emb,
+                         long long R, const long long* t, const float* z, long long B, bool gen, bool disc) {
+  GatherParams gp{};
+  gp.node_emb = node_emb; gp.rel_emb = rel_emb; gp.N = N; gp.R = R; gp.E = c->dims.embed_dim; gp.Z = c->dims.noise_dim;
+  gp.heads = t; gp.rels = t + 1; gp.tails = t + 2; gp.head_stride = gp.rel_stride = gp.tail_stride = 3;
+  gp.z = z;
+  gp.xg = gen ? st.xg0 : nullptr; gp.ldg = c->kg0p;
+  gp.xd = disc ? st.xd0 : nullptr; gp.ldd = c->kd0p;
+  gp.B = B; gp.err_flag = c->err_flag;
+  return gp;
+}
+
+// The pass over staged slot `slot` that produces the requested results; the slot must hold the operands they need.
+int staged_pass(pbg_ctx* c, int slot, void* gen_out, int out_dtype, float* gen_scores, float* logits, float* probs,
+                void* stream, Pass& a) {
+  if (slot < 0 || slot > 1) return fail(c, PBG_ERR_INVALID, "score_staged: slot must be 0 or 1");
+  const StageSlot& st = c->stage[slot];
+  if (st.B <= 0) return fail(c, PBG_ERR_INVALID, "score_staged: nothing staged in slot %d", slot);
+  a.gen_out = gen_out; a.out_dtype = out_dtype; a.gen_scores = gen_scores; a.logits = logits; a.probs = probs;
+  a.run_g = (gen_out != nullptr || gen_scores != nullptr); a.run_d = (logits != nullptr);
+  if (a.run_g && !st.has_g) return fail(c, PBG_ERR_INVALID, "score_staged: slot %d holds no generator operands", slot);
+  if (a.run_d && !st.has_d) return fail(c, PBG_ERR_INVALID, "score_staged: slot %d holds no discriminator operands", slot);
+  a.B = st.B; a.prec = PBG_PREC_BF16; a.stream = (cudaStream_t)stream;
+  return PBG_OK;
+}
+}  // namespace
+
 int pbg_stage_triplets(pbg_ctx* c, int slot, const float* node_emb, int64_t N, const float* rel_emb, int64_t R,
                        const int64_t* triplets, const float* z, int64_t B, int want_gen, int want_disc, void* stream) {
   if (!c) return PBG_ERR_INVALID;
@@ -1228,13 +1235,7 @@ int pbg_stage_triplets(pbg_ctx* c, int slot, const float* node_emb, int64_t N, c
   }
   const long long* t = (const long long*)triplets;
   StageParams sp{};
-  GatherParams& gp = sp.g;
-  gp.node_emb = node_emb; gp.rel_emb = rel_emb; gp.N = N; gp.R = R; gp.E = c->dims.embed_dim; gp.Z = c->dims.noise_dim;
-  gp.heads = t; gp.rels = t + 1; gp.tails = t + 2; gp.head_stride = gp.rel_stride = gp.tail_stride = 3;
-  gp.z = z;
-  gp.xg = want_gen ? st.xg0 : nullptr; gp.ldg = c->kg0p;
-  gp.xd = want_disc ? st.xd0 : nullptr; gp.ldd = c->kd0p;
-  gp.B = B; gp.err_flag = c->err_flag;
+  sp.g = slot_gather(c, st, node_emb, N, rel_emb, R, t, z, B, want_gen != 0, want_disc != 0);
   sp.xt = want_gen ? st.xt : nullptr;
   const int blocks = (int)std::min<long long>((B + 3) / 4, (long long)c->num_sms * 16);
   { LaunchScope ls(c, PBG_K_GATHER, s);
@@ -1248,42 +1249,29 @@ int pbg_stage_triplets(pbg_ctx* c, int slot, const float* node_emb, int64_t N, c
 int pbg_score_staged(pbg_ctx* c, int slot, void* gen_out, int out_dtype, float* gen_scores, float* logits, float* probs,
                      void* stream) {
   if (!c) return PBG_ERR_INVALID;
-  if (slot < 0 || slot > 1) return fail(c, PBG_ERR_INVALID, "score_staged: slot must be 0 or 1");
-  const StageSlot& st = c->stage[slot];
-  if (st.B <= 0) return fail(c, PBG_ERR_INVALID, "score_staged: nothing staged in slot %d", slot);
   Pass a;
-  a.gen_out = gen_out; a.out_dtype = out_dtype; a.gen_scores = gen_scores; a.logits = logits; a.probs = probs;
-  a.run_g = (gen_out != nullptr || gen_scores != nullptr); a.run_d = (logits != nullptr);
-  if (a.run_g && !st.has_g) return fail(c, PBG_ERR_INVALID, "score_staged: slot %d holds no generator operands", slot);
-  if (a.run_d && !st.has_d) return fail(c, PBG_ERR_INVALID, "score_staged: slot %d holds no discriminator operands", slot);
+  PBG_TRY(staged_pass(c, slot, gen_out, out_dtype, gen_scores, logits, probs, stream, a));
   if (!a.run_g && !a.run_d) return PBG_OK;
-  a.B = st.B; a.prec = PBG_PREC_BF16; a.stream = (cudaStream_t)stream;
   PBG_CUDA(c, cudaSetDevice(c->dims.device));
-  PBG_TRY(ensure_ws(c, PBG_PREC_BF16, st.B, a.stream));
+  PBG_TRY(ensure_ws(c, PBG_PREC_BF16, a.B, a.stream));
   GatherParams gp{};
-  return launch_pass2(c, c->ws_bf16, a, gp, 0, st.B, gen_out, gen_scores, true, &st);
+  return launch_pass2(c, c->ws_bf16, a, gp, 0, a.B, gen_out, gen_scores, true, &c->stage[slot]);
 }
 
 int pbg_score_staged_stage_next(pbg_ctx* c, int slot, void* gen_out, int out_dtype, float* gen_scores, float* logits, float* probs,
                                 const float* node_emb, int64_t N, const float* rel_emb, int64_t R, const int64_t* next_triplets,
                                 const float* next_z, int64_t next_B, void* stream) {
   if (!c) return PBG_ERR_INVALID;
-  if (slot < 0 || slot > 1) return fail(c, PBG_ERR_INVALID, "score_staged: slot must be 0 or 1");
+  Pass a;
+  PBG_TRY(staged_pass(c, slot, gen_out, out_dtype, gen_scores, logits, probs, stream, a));
   StageSlot& st = c->stage[slot];
   StageSlot& nx = c->stage[1 - slot];
-  if (st.B <= 0) return fail(c, PBG_ERR_INVALID, "score_staged: nothing staged in slot %d", slot);
   if (next_B <= 0 || next_B > kMaxChunk) return fail(c, PBG_ERR_INVALID, "stage next: B must be in [1, %lld]", kMaxChunk);
   if (!node_emb || !rel_emb || !next_triplets) return fail(c, PBG_ERR_INVALID, "null tensor");
-  Pass a;
-  a.gen_out = gen_out; a.out_dtype = out_dtype; a.gen_scores = gen_scores; a.logits = logits; a.probs = probs;
-  a.run_g = (gen_out != nullptr || gen_scores != nullptr); a.run_d = (logits != nullptr);
-  if (a.run_g && !st.has_g) return fail(c, PBG_ERR_INVALID, "score_staged: slot %d holds no generator operands", slot);
-  if (a.run_d && !st.has_d) return fail(c, PBG_ERR_INVALID, "score_staged: slot %d holds no discriminator operands", slot);
   if (!a.run_g && !a.run_d) return fail(c, PBG_ERR_INVALID, "score_staged_stage_next: no result requested");
   if (a.run_g && !next_z && !c->lat_on) return fail(c, PBG_ERR_INVALID, "generator needs latents z");
-  a.B = st.B; a.prec = PBG_PREC_BF16; a.stream = (cudaStream_t)stream;
   PBG_CUDA(c, cudaSetDevice(c->dims.device));
-  PBG_TRY(ensure_ws(c, PBG_PREC_BF16, st.B, a.stream));
+  PBG_TRY(ensure_ws(c, PBG_PREC_BF16, a.B, a.stream));
   PBG_TRY(ensure_stage(c, nx, next_B, a.stream));
   if (a.run_g && !next_z) {   // drawn now, ahead of the pass that gathers it: stream order is staging order
     PBG_TRY(draw_stream(c, next_B, nx.z, a.stream));
@@ -1291,14 +1279,8 @@ int pbg_score_staged_stage_next(pbg_ctx* c, int slot, void* gen_out, int out_dty
   }
   // the next request gets the operands this pass produces results for (same models in flight)
   const long long* t = reinterpret_cast<const long long*>(next_triplets);
-  GatherParams gp{};
-  gp.node_emb = node_emb; gp.rel_emb = rel_emb; gp.N = N; gp.R = R; gp.E = c->dims.embed_dim; gp.Z = c->dims.noise_dim;
-  gp.heads = t; gp.rels = t + 1; gp.tails = t + 2; gp.head_stride = gp.rel_stride = gp.tail_stride = 3;
-  gp.z = next_z;
-  gp.xg = a.run_g ? nx.xg0 : nullptr; gp.ldg = c->kg0p;
-  gp.xd = a.run_d ? nx.xd0 : nullptr; gp.ldd = c->kd0p;
-  gp.B = next_B; gp.err_flag = c->err_flag;
-  PBG_TRY(launch_pass2(c, c->ws_bf16, a, gp, 0, st.B, gen_out, gen_scores, true, &st, true));
+  const GatherParams gp = slot_gather(c, nx, node_emb, N, rel_emb, R, t, next_z, next_B, a.run_g, a.run_d);
+  PBG_TRY(launch_pass2(c, c->ws_bf16, a, gp, 0, a.B, gen_out, gen_scores, true, &st, true));
   st.B = -1;   // consumed (with the workspace discard on its rows are dropped from L2 as the first layers finish with them)
   nx.B = next_B; nx.has_g = a.run_g; nx.has_d = a.run_d; nx.has_xt = false;
   nx.node_emb = node_emb; nx.N = N; nx.tails = t + 2;
@@ -1318,20 +1300,15 @@ int pbg_linear_bf16(pbg_ctx* c, int model, int layer, const void* a, void* out, 
   // ONE layer of the product kernel: the pass kernel with a single item kind, its A operand the caller's matrix and no
   // dependency to wait for; the layer's own epilogue (LeakyReLU store / row dot + sigmoid / tanh) writes `out`.
   static const int kind_of[2][3] = {{IT_G_L0, IT_G_L1, IT_G_L2}, {IT_D_L0, IT_D_L1, -1}};
-  static const int epi_of[5] = {PEPI_STORE, PEPI_STORE, PEPI_STORE, PEPI_ROWDOT, PEPI_TANH};
-  static const int pred_of[5] = {DEP_X, DEP_X, DEP_G0, DEP_D0, DEP_G1};
-  static const int out_of[5] = {DEP_G0, DEP_D0, DEP_G1, -1, -1};
   const int k = kind_of[model][layer];
   const Linear& l = model == 0 ? c->g[layer] : c->d[layer];
-  const int bn = (l.np % 256 == 0) ? 256 : 128;
+  const bool store = kEpiOf[k] == PEPI_STORE;
+  CUtensorMap amap, omap;
+  PBG_TRY(make_tmap(c, &amap, a, M, l.kp, kBlockM));
+  if (store) PBG_TRY(make_tmap(c, &omap, out, M, l.np, 32));
   Pass2Params p;
   memset(&p, 0, sizeof p);
-  PBG_TRY(make_tmap(c, &p.tm_a[k], a, M, l.kp, kBlockM));
-  p.tm_w[k] = bn == 256 ? l.tmap_w128 : l.tmap_w64;
-  if (epi_of[k] == PEPI_STORE) PBG_TRY(make_tmap(c, &p.tm_o[k], out, M, l.np, 32));
-  p.layer[k] = P2Layer{l.kp / kBlockK, bn, l.np / bn, epi_of[k], pred_of[k], out_of[k], l.np, -1, l.b_pad,
-                       epi_of[k] == PEPI_STORE ? static_cast<__nv_bfloat16*>(out) : nullptr};
-  p.layer_mask = 1u << k;
+  set_layer(p, k, l, amap, store ? &omap : nullptr, store ? static_cast<__nv_bfloat16*>(out) : nullptr, l.np);
   const int nrb = static_cast<int>((M + kP2Rows - 1) / kP2Rows);
   p.seg[0] = P2Segment{k, p.layer[k].n_tiles, 0, 0, k, 0};
   p.n_seg = 1; p.n_total = nrb * p.layer[k].n_tiles;
@@ -1352,7 +1329,7 @@ int pbg_linear_bf16(pbg_ctx* c, int model, int layer, const void* a, void* out, 
   const int grid = pass_grid(c) & ~1;
   cudaError_t le;
   { LaunchScope ls(c, model == 0 ? PBG_K_G_L0 + layer : PBG_K_D_L0 + layer, s);
-    le = launch_p2<false, false, false>(c, p, grid, s, false); }
+    le = launch_pdl(false, kPass2[0], grid, kP2Threads, P2Smem::kTotal, s, p); }
   if (le == cudaSuccess) le = cudaGetLastError();
   if (le != cudaSuccess) return fail(c, PBG_ERR_CUDA, "single-layer pass launch failed: %s", cudaGetErrorString(le));
   return PBG_OK;
@@ -1434,47 +1411,45 @@ int score_host(pbg_ctx* c, const float* node_emb, int64_t N, const float* rel_em
   if (run_g && !z_host && !c->lat_on) return fail(c, PBG_ERR_INVALID, "generator needs latents z");
   PBG_CUDA(c, cudaSetDevice(c->dims.device));
   const int E = c->dims.embed_dim, Z = c->dims.noise_dim;
+  cudaStream_t s = c->own_stream;
   if (c->host_cap < B) {
-    PBG_CUDA(c, cudaDeviceSynchronize());
-    cudaFree(c->st_block); c->st_block = nullptr; c->host_cap = 0;
+    PBG_TRY(begin_growth(c, s, "the host staging block"));
+    c->host_cap = 0;
     const size_t per_row = sizeof(long long) * 3 + sizeof(float) * (Z + 3 + E);
-    PBG_CUDA(c, cudaMalloc(&c->st_block, per_row * B + 64));   // + alignment padding in front of z and gen_out
+    PBG_TRY(realloc_dev(c, c->st_block, per_row * B + 64));   // + alignment padding in front of z and gen_out
     c->host_cap = B;
   }
-  {
-    // one device block, laid out for THIS call's B: [triplets | z | scores | logits | probs | gen_out]; z and gen_out rows
-    // are read / written with 16-byte vectors, so their offsets are rounded up
-    auto up16 = [](size_t v) { return (v + 15) & ~static_cast<size_t>(15); };
-    char* b0 = c->st_block;
-    size_t off = 0;
-    c->st_trip = reinterpret_cast<long long*>(b0 + off);  off = up16(off + sizeof(long long) * 3 * B);
-    c->st_z = reinterpret_cast<float*>(b0 + off);         off += sizeof(float) * Z * B;
-    c->st_scores = reinterpret_cast<float*>(b0 + off);    off += sizeof(float) * B;
-    c->st_logits = reinterpret_cast<float*>(b0 + off);    off += sizeof(float) * B;
-    c->st_probs = reinterpret_cast<float*>(b0 + off);     off = up16(off + sizeof(float) * B);
-    c->st_gen = reinterpret_cast<float*>(b0 + off);
-  }
-  cudaStream_t s = c->own_stream;
+  // one device block, laid out for THIS call's B: [triplets | z | scores | logits | probs | gen_out]; z and gen_out rows
+  // are read / written with 16-byte vectors, so their offsets are rounded up
+  auto up16 = [](size_t v) { return (v + 15) & ~static_cast<size_t>(15); };
+  char* b0 = c->st_block;
+  size_t off = 0;
+  long long* trip = reinterpret_cast<long long*>(b0 + off);  off = up16(off + sizeof(long long) * 3 * B);
+  float* z = reinterpret_cast<float*>(b0 + off);             off += sizeof(float) * Z * B;
+  float* scores = reinterpret_cast<float*>(b0 + off);        off += sizeof(float) * B;
+  float* logits = reinterpret_cast<float*>(b0 + off);        off += sizeof(float) * B;
+  float* probs = reinterpret_cast<float*>(b0 + off);         off = up16(off + sizeof(float) * B);
+  float* gen = reinterpret_cast<float*>(b0 + off);
   // every DMA operation costs a few microseconds of set-up beside its bytes (six of them were a third of a 4096-triplet
   // call): the packed form moves [triplets | z] and [scores | logits | probs] in one copy each
-  const bool one_h2d = packed && z_host && reinterpret_cast<char*>(c->st_z) == reinterpret_cast<char*>(c->st_trip) + sizeof(long long) * 3 * B;
+  const bool one_h2d = packed && z_host && reinterpret_cast<char*>(z) == reinterpret_cast<char*>(trip) + sizeof(long long) * 3 * B;
   if (one_h2d) {
-    PBG_CUDA(c, cudaMemcpyAsync(c->st_trip, triplets_host, sizeof(long long) * 3 * B + sizeof(float) * Z * B, cudaMemcpyHostToDevice, s));
+    PBG_CUDA(c, cudaMemcpyAsync(trip, triplets_host, sizeof(long long) * 3 * B + sizeof(float) * Z * B, cudaMemcpyHostToDevice, s));
   } else {
-    PBG_CUDA(c, cudaMemcpyAsync(c->st_trip, triplets_host, sizeof(long long) * 3 * B, cudaMemcpyHostToDevice, s));
-    if (run_g && z_host) PBG_CUDA(c, cudaMemcpyAsync(c->st_z, z_host, sizeof(float) * Z * B, cudaMemcpyHostToDevice, s));
+    PBG_CUDA(c, cudaMemcpyAsync(trip, triplets_host, sizeof(long long) * 3 * B, cudaMemcpyHostToDevice, s));
+    if (run_g && z_host) PBG_CUDA(c, cudaMemcpyAsync(z, z_host, sizeof(float) * Z * B, cudaMemcpyHostToDevice, s));
   }
-  PBG_TRY(pbg_score_triplets(c, node_emb, N, rel_emb, R, (const int64_t*)c->st_trip, run_g && z_host ? c->st_z : nullptr,
-                             gen_out_host ? c->st_gen : nullptr, PBG_DT_F32, gen_scores_host ? c->st_scores : nullptr,
-                             logits_host ? c->st_logits : nullptr, probs_host ? c->st_probs : nullptr, B, precision, s));
+  PBG_TRY(pbg_score_triplets(c, node_emb, N, rel_emb, R, (const int64_t*)trip, run_g && z_host ? z : nullptr,
+                             gen_out_host ? gen : nullptr, PBG_DT_F32, gen_scores_host ? scores : nullptr,
+                             logits_host ? logits : nullptr, probs_host ? probs : nullptr, B, precision, s));
   if (packed) {
-    PBG_CUDA(c, cudaMemcpyAsync(gen_scores_host, c->st_scores, sizeof(float) * 3 * B, cudaMemcpyDeviceToHost, s));
+    PBG_CUDA(c, cudaMemcpyAsync(gen_scores_host, scores, sizeof(float) * 3 * B, cudaMemcpyDeviceToHost, s));
   } else {
-    if (gen_scores_host) PBG_CUDA(c, cudaMemcpyAsync(gen_scores_host, c->st_scores, sizeof(float) * B, cudaMemcpyDeviceToHost, s));
-    if (logits_host) PBG_CUDA(c, cudaMemcpyAsync(logits_host, c->st_logits, sizeof(float) * B, cudaMemcpyDeviceToHost, s));
-    if (probs_host) PBG_CUDA(c, cudaMemcpyAsync(probs_host, c->st_probs, sizeof(float) * B, cudaMemcpyDeviceToHost, s));
+    if (gen_scores_host) PBG_CUDA(c, cudaMemcpyAsync(gen_scores_host, scores, sizeof(float) * B, cudaMemcpyDeviceToHost, s));
+    if (logits_host) PBG_CUDA(c, cudaMemcpyAsync(logits_host, logits, sizeof(float) * B, cudaMemcpyDeviceToHost, s));
+    if (probs_host) PBG_CUDA(c, cudaMemcpyAsync(probs_host, probs, sizeof(float) * B, cudaMemcpyDeviceToHost, s));
   }
-  if (gen_out_host) PBG_CUDA(c, cudaMemcpyAsync(gen_out_host, c->st_gen, sizeof(float) * E * B, cudaMemcpyDeviceToHost, s));
+  if (gen_out_host) PBG_CUDA(c, cudaMemcpyAsync(gen_out_host, gen, sizeof(float) * E * B, cudaMemcpyDeviceToHost, s));
   return pbg_check_indices(c, s);  // one sync: results + the out-of-range flag
 }
 }  // namespace
