@@ -62,7 +62,12 @@ typedef struct pbg_dims {
 int pbg_abi_version(void);
 
 /* Replaces `Generator(E, Z).to(device)` / `Discriminator(E, H).to(device)`
- * (pro_b_gan_infer.py:93-94): allocates the device-side state for one model pair. */
+ * (pro_b_gan_infer.py:93-94): allocates the device-side state for one model pair.
+ * Accepts embed_dim, noise_dim and g_hidden that are multiples of 8, d_hidden a multiple of 16 and
+ * leaky_slope in [0, 1]; anything else is PBG_ERR_UNSUPPORTED.  bf16 mode has two further limits,
+ * checked at launch (PBG_ERR_UNSUPPORTED, the ctx stays usable): a pass that runs the generator needs
+ * embed_dim <= 512, and a pass that runs the discriminator needs d_hidden <= 8192 (d_hidden / 2
+ * rounded up to 128 is at most 4096).  fp32 mode has neither limit. */
 int pbg_create(pbg_ctx** out, const pbg_dims* dims);
 void pbg_destroy(pbg_ctx* ctx);
 

@@ -1023,7 +1023,9 @@ pbg_pass2_kernel(const __grid_constant__ Pass2Params p) {
                 }
               }
             }
-            if (bulk_mirror) {
+            // bulk_mirror implies embed_dim % 64 == 0, so a chunk is wholly valid or wholly padding; a padding chunk
+            // (E = 64, 192, 320, ...) has nothing to mirror, and its 128 bytes would land on the next row
+            if (bulk_mirror && col0 < p.n_valid) {
               uint8_t* myrow = st + lane * 128;   // only this lane writes and (through its bulk stores) reads it
               const int rounds = p.out_f32 ? 2 : 1;
               for (int rd = 0; rd < rounds; ++rd) {
