@@ -76,7 +76,9 @@ struct Workspace {
 struct TopkState {
   const float* table = nullptr; long long N = 0, n_pad = 0;
   __nv_bfloat16* tn = nullptr; float* inv_t = nullptr; CUtensorMap tm_t;
+  unsigned* err_t = nullptr;   // the table's largest bf16 rounding error (float bits; topk_kernel.cuh: tk_err)
   long long q_cap = 0; __nv_bfloat16* qn = nullptr; float* inv_q = nullptr; CUtensorMap tm_q;
+  float* err_q = nullptr;      // [q_cap] each query row's bf16 rounding error (filter path: topk_tau_kernel)
   size_t cand_cap = 0; unsigned* cand_grp = nullptr; unsigned* cand_mask = nullptr; int* cand_cnt = nullptr;   // [rows][lists][kTkCand]
   size_t samp_cap = 0; int* samp_keys = nullptr;   // [rows][sample lists][kTkKeys]
   float* tau = nullptr; int* flag = nullptr;       // [q_cap]
@@ -729,13 +731,15 @@ int pbg_topk_prepare(pbg_ctx* c, const float* table, int64_t N, void* stream) {
     t.n_pad = 0;
     PBG_TRY(realloc_dev(c, t.tn, sizeof(__nv_bfloat16) * n_pad * E));
     PBG_TRY(realloc_dev(c, t.inv_t, sizeof(float) * n_pad));
+    if (!t.err_t) PBG_TRY(realloc_dev(c, t.err_t, sizeof(unsigned)));
     t.n_pad = n_pad;
     if (E == 128) PBG_TRY(make_tmap(c, &t.tm_t, t.tn, n_pad, E, 128));
   }
   t.table = table; t.N = N;
+  PBG_CUDA(c, cudaMemsetAsync(t.err_t, 0, sizeof(unsigned), s));
   { LaunchScope ls(c, PBG_K_OTHER, s);
-    if (E <= 128) topk_prepare_kernel<8, 1><<<c->num_sms * 8, 256, 0, s>>>(table, N, n_pad, E, t.tn, t.inv_t);
-    else topk_prepare_kernel<2, 4><<<c->num_sms * 8, 256, 0, s>>>(table, N, n_pad, E, t.tn, t.inv_t); }
+    if (E <= 128) topk_prepare_kernel<8, 1, true><<<c->num_sms * 8, 256, 0, s>>>(table, N, n_pad, E, t.tn, t.inv_t, t.err_t);
+    else topk_prepare_kernel<2, 4, true><<<c->num_sms * 8, 256, 0, s>>>(table, N, n_pad, E, t.tn, t.inv_t, t.err_t); }
   PBG_CUDA(c, cudaGetLastError());
   return PBG_OK;
 }
@@ -813,6 +817,7 @@ int pbg_topk(pbg_ctx* c, const float* queries, int64_t B, int k, int64_t* out_id
       t.q_cap = 0;
       PBG_TRY(realloc_dev(c, t.qn, sizeof(__nv_bfloat16) * rows_pad * E));
       PBG_TRY(realloc_dev(c, t.inv_q, sizeof(float) * rows_pad));
+      PBG_TRY(realloc_dev(c, t.err_q, sizeof(float) * rows_pad));
       PBG_TRY(realloc_dev(c, t.flag, sizeof(int) * rows_pad));
       PBG_TRY(realloc_dev(c, t.tau, sizeof(float) * rows_pad));
       t.q_cap = rows_pad;
@@ -820,8 +825,8 @@ int pbg_topk(pbg_ctx* c, const float* queries, int64_t B, int k, int64_t* out_id
     }
     { LaunchScope ls(c, PBG_K_OTHER, s);
       const unsigned pg = static_cast<unsigned>(std::min<long long>(c->num_sms * 8, (rows_pad + 7) / 8));
-      if (E <= 128) topk_prepare_kernel<8, 1><<<pg, 256, 0, s>>>(q, rows, rows_pad, E, t.qn, t.inv_q);
-      else topk_prepare_kernel<2, 4><<<pg, 256, 0, s>>>(q, rows, rows_pad, E, t.qn, t.inv_q); }
+      if (E <= 128) topk_prepare_kernel<8, 1, false><<<pg, 256, 0, s>>>(q, rows, rows_pad, E, t.qn, t.inv_q, nullptr);
+      else topk_prepare_kernel<2, 4, false><<<pg, 256, 0, s>>>(q, rows, rows_pad, E, t.qn, t.inv_q, nullptr); }
     PBG_CUDA(c, cudaGetLastError());
     long long* oi = reinterpret_cast<long long*>(out_idx) + off * k;
     float* os = out_scores + off * k;
@@ -874,12 +879,13 @@ int pbg_topk(pbg_ctx* c, const float* queries, int64_t B, int k, int64_t* out_id
     { LaunchScope ls(c, PBG_K_TOPK, s);
       PBG_CUDA(c, launch_pdl(true, pbg_topk_scan_kernel<TK_SAMPLE>, std::min(grid, 2 * ((ps.total + ps.span - 1) / ps.span)), kPassThreads, TkSmem::kTotal, s, ps)); }
     { LaunchScope ls(c, PBG_K_OTHER, s);
-      PBG_CUDA(c, launch_pdl(false, topk_tau_kernel, static_cast<unsigned>((rows_pad + 7) / 8), 256, 0, s, t.samp_keys, n_slists, rows, rows_pad, k, t.tau)); }
+      PBG_CUDA(c, launch_pdl(false, topk_tau_kernel, static_cast<unsigned>((rows_pad + 7) / 8), 256, 0, s, t.samp_keys, n_slists, rows, rows_pad, k,
+                             q, t.inv_q, t.qn, t.err_q, t.err_t, t.tau)); }
     { LaunchScope ls(c, PBG_K_TOPK, s);
       PBG_CUDA(c, launch_pdl(true, pbg_topk_scan_kernel<TK_SCAN>, std::min(grid, 2 * ((pm.total + pm.span - 1) / pm.span)), kPassThreads, TkSmem::kTotal, s, pm)); }
     { LaunchScope ls(c, PBG_K_OTHER, s);
       PBG_CUDA(c, launch_pdl(false, topk_rescore_kernel, static_cast<unsigned>((rows + kTkRescoreWarps - 1) / kTkRescoreWarps), 32 * kTkRescoreWarps, 0, s,
-                             q, t.inv_q, t.table, t.inv_t, t.cand_grp, t.cand_mask, t.cand_cnt, t.tau, n_lists, rows, t.N, k, oi, os, t.flag)); }
+                             q, t.inv_q, t.table, t.inv_t, t.cand_grp, t.cand_mask, t.cand_cnt, t.tau, t.err_q, t.err_t, n_lists, rows, t.N, k, oi, os, t.flag)); }
     { // rows the filter could not prove: exact scan, one CTA per row (rare)
       LaunchScope ls(c, PBG_K_OTHER, s);
       PBG_CUDA(c, launch_pdl(true, topk_exact_kernel, static_cast<unsigned>(std::min<long long>(rows, 2ll * c->num_sms)), 256,
@@ -1027,7 +1033,7 @@ void pbg_destroy(pbg_ctx* c) {
   free_stage(c->stage[0]); free_stage(c->stage[1]);
   cudaFree(c->err_flag); cudaFree(c->trace);
   cudaFree(c->lat_st); cudaFree(c->lat_z);
-  cudaFree(c->tk.tn); cudaFree(c->tk.inv_t); cudaFree(c->tk.qn); cudaFree(c->tk.inv_q);
+  cudaFree(c->tk.tn); cudaFree(c->tk.inv_t); cudaFree(c->tk.err_t); cudaFree(c->tk.qn); cudaFree(c->tk.inv_q); cudaFree(c->tk.err_q);
   cudaFree(c->tk.cand_grp); cudaFree(c->tk.cand_mask); cudaFree(c->tk.cand_cnt); cudaFree(c->tk.flag);
   cudaFree(c->tk.samp_keys); cudaFree(c->tk.tau); cudaFree(c->tk.score_buf);
 

@@ -43,10 +43,18 @@ inline int tk_sample_stride(int k) { return k <= 16 ? 4 : 2; }
 constexpr int kTkKeys = 16;           // best group keys a thread keeps per sample list; a row's lists together hold >= 2 k keys (pbg.cu: chunk size)
 constexpr int kTkRescoreMax = 1024;   // candidates per row the rescoring kernel takes (about 8 k + a dozen arrive); more: exact scan
 constexpr int kTkRescoreWarps = 4;    // rows per rescoring CTA (32 KB of candidate scores / indices in shared memory)
-// |bf16 score - exact score| for unit vectors: both operands rounded to 8 significant bits (relative 2^-9 each) give
-// (2^-8 + 2^-18) * sum |q_i t_i| <= 0.003910 by Cauchy-Schwarz; + fp32 accumulation of 128 exact products (<= 1.5e-5)
-// + the sample keys' 5 truncated mantissa bits (<= 4e-6) = 0.00393; the rest is slack
-constexpr float kTkErrBound = 0.0045f;
+// |bf16 score - exact score| for unit vectors q, t and their bf16 copies q', t' (round to nearest, 8 significant bits:
+// relative error up to 2^-8 per entry, so a fixed constant would have to be (2^-7 + 2^-16) * sum |q_i t_i| <= 0.0079):
+//   |q'.t' - q.t| <= ||q' - q|| * ||t'|| + ||q|| * ||t' - t|| <= e_q (1 + e_t) + e_t
+// with e_q = ||q' - q|| of the query row (measured by topk_tau_kernel) and e_t the largest ||t' - t|| of the table
+// (measured by topk_prepare_kernel); + fp32 accumulation of 128 products in the tensor cores and in the rescoring
+// (<= 1.5e-5) + the sample keys' 5 truncated mantissa bits (<= 4e-6).  Random rows give e_q ~ 0.0017, e_t ~ 0.0023
+// (err ~ 0.0040); rows whose entries all sit just past a power of two reach 2^-8 * ||x|| and err ~ 0.0078.
+constexpr float kTkErrSlack = 2e-5f;
+__device__ __forceinline__ float tk_err(float e_q, const unsigned* err_t) {
+  const float e_t = __uint_as_float(*err_t);
+  return e_q * (1.f + e_t) + e_t + kTkErrSlack;
+}
 enum : int { TK_SAMPLE = 0, TK_SCAN = 1 };
 
 struct alignas(64) TopkParams {
@@ -103,16 +111,32 @@ __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;"
 // padding rows are zero.  HBM-bound (E fp32 in, E bf16 + 4 B out per row): a warp takes R rows per iteration, every
 // load of those rows in flight before the first reduction (bytes in flight per SM, not instruction count, set the rate),
 // and keeps the values in registers for the scaling pass.  <R = 8, V = 1>: E <= 128; <R = 2, V = 4>: E <= 512 in
-// registers, wider rows are read a second time.
-template <int R, int V>
+// registers, wider rows are read a second time.  ERR (the table): the largest row rounding error ||bf16(x * inv) -
+// x * inv||_2 (the error bound above) goes to *err_max -- non-negative floats order like their bits, the caller zeroes
+// the word.  The queries' errors are measured by topk_tau_kernel, off this kernel's critical path.
+__device__ __forceinline__ float tk_store_bf16(__nv_bfloat16* dst, float4 v) {   // returns the squared rounding error
+  const __nv_bfloat162 lo = __floats2bfloat162_rn(v.x, v.y), hi = __floats2bfloat162_rn(v.z, v.w);
+  const float2 rl = __bfloat1622float2(lo), rh = __bfloat1622float2(hi);
+  uint2 w;
+  w.x = *reinterpret_cast<const uint32_t*>(&lo);
+  w.y = *reinterpret_cast<const uint32_t*>(&hi);
+  *reinterpret_cast<uint2*>(dst) = w;
+  const float a = v.x - rl.x, b = v.y - rl.y, c = v.z - rh.x, d = v.w - rh.y;   // exact: x minus its rounding
+  return a * a + b * b + c * c + d * d;
+}
+
+template <int R, int V, bool ERR>
 __global__ void __launch_bounds__(256) topk_prepare_kernel(const float* __restrict__ x, long long rows, long long rows_pad, int E,
-                                                           __nv_bfloat16* __restrict__ xn, float* __restrict__ inv) {
+                                                           __nv_bfloat16* __restrict__ xn, float* __restrict__ inv,
+                                                           unsigned* __restrict__ err_max) {
   pdl_wait();
   const int lane = threadIdx.x & 31;
   const long long warp0 = (static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
   const long long nwarp = (static_cast<long long>(gridDim.x) * blockDim.x) >> 5;
   const bool in_regs = E <= 128 * V;
+  float emax = 0.f;   // ERR: this warp's largest row error
   for (long long r0 = warp0 * R; r0 < rows_pad; r0 += nwarp * R) {
+    float es[R];
     float4 v[R][V];
     float ss[R];
 #pragma unroll
@@ -146,6 +170,7 @@ __global__ void __launch_bounds__(256) topk_prepare_kernel(const float* __restri
 #pragma unroll
     for (int i = 0; i < R; ++i) {
       const long long r = r0 + i;
+      es[i] = 0.f;
       if (r >= rows_pad) continue;
       if (r >= rows) {
         for (int c = lane * 4; c < E; c += 128) store4<__nv_bfloat16>(xn + r * E + c, make_float4(0.f, 0.f, 0.f, 0.f));
@@ -157,16 +182,28 @@ __global__ void __launch_bounds__(256) topk_prepare_kernel(const float* __restri
 #pragma unroll
         for (int j = 0; j < V; ++j) {
           const int c = lane * 4 + j * 128;
-          if (c < E) store4<__nv_bfloat16>(xn + r * E + c, make_float4(v[i][j].x * iv, v[i][j].y * iv, v[i][j].z * iv, v[i][j].w * iv));
+          const float4 y = make_float4(v[i][j].x * iv, v[i][j].y * iv, v[i][j].z * iv, v[i][j].w * iv);
+          if (c < E) { if (ERR) es[i] += tk_store_bf16(xn + r * E + c, y); else store4<__nv_bfloat16>(xn + r * E + c, y); }
         }
       } else {
         for (int c = lane * 4; c < E; c += 128) {
           const float4 w = *reinterpret_cast<const float4*>(x + r * E + c);
-          store4<__nv_bfloat16>(xn + r * E + c, make_float4(w.x * iv, w.y * iv, w.z * iv, w.w * iv));
+          const float4 y = make_float4(w.x * iv, w.y * iv, w.z * iv, w.w * iv);
+          if (ERR) es[i] += tk_store_bf16(xn + r * E + c, y); else store4<__nv_bfloat16>(xn + r * E + c, y);
         }
       }
     }
+    if (ERR) {
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) {
+#pragma unroll
+        for (int i = 0; i < R; ++i) es[i] += __shfl_xor_sync(0xffffffffu, es[i], o);
+      }
+#pragma unroll
+      for (int i = 0; i < R; ++i) emax = fmaxf(emax, sqrtf(es[i]));
+    }
   }
+  if (ERR && lane == 0 && emax > 0.f) atomicMax(err_max, __float_as_uint(emax));
   pdl_launch_dependents();   // at the END: successors released at entry sit beside this kernel's blocks and slow them
 }
 
@@ -388,12 +425,15 @@ pbg_topk_scan_kernel(const __grid_constant__ TopkParams p) {
 
 // One warp per query row: s_k = the k-th largest of the row's sampled group keys (n_lists x kTkKeys of them) with its
 // position bits cleared -- at least k sampled entities have a bf16 score >= s_k, hence an exact score >= s_k - err, so
-// the k-th exact score of the row is >= s_k - err.  The scan's cut-off is tau = s_k - 2 err - 1e-4: every entity that is
-// NOT marked has a bf16 score <= tau, i.e. an exact score <= tau + err < s_k - err <= the k-th exact score -- the proof
-// obligation of the rescoring kernel holds by construction (it is still checked), at the price of about a dozen more
-// candidates per row than a cut-off at s_k itself.  Fewer than k positive keys: tau = 0.
+// the k-th exact score of the row is >= s_k - err (err = tk_err of the row).  The scan's cut-off is tau = s_k - 2 err -
+// 1e-4: every entity that is NOT marked has a bf16 score <= tau, i.e. an exact score <= tau + err < s_k - err <= the k-th
+// exact score -- the proof obligation of the rescoring kernel holds by construction (it is still checked), at the price
+// of about a dozen more candidates per row than a cut-off at s_k itself.  Fewer than k positive keys: tau = 0.
+// The row's e_q is measured here (E = 128: 4 dimensions per lane) and kept in err_q[row] for the rescoring kernel.
 __global__ void __launch_bounds__(256) topk_tau_kernel(const int* __restrict__ samp_keys, int n_lists, long long B, long long rows_pad,
-                                                       int k, float* __restrict__ tau) {
+                                                       int k, const float* __restrict__ q, const float* __restrict__ inv_q,
+                                                       const __nv_bfloat16* __restrict__ qn, float* __restrict__ err_q,
+                                                       const unsigned* __restrict__ err_t, float* __restrict__ tau) {
   pdl_wait();
   const int lane = threadIdx.x & 31;
   const long long row = (static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x) >> 5;
@@ -403,6 +443,20 @@ __global__ void __launch_bounds__(256) topk_tau_kernel(const int* __restrict__ s
   int mine[kTkKeys];
 #pragma unroll
   for (int i = 0; i < kTkKeys; ++i) { const int c = i * 32 + lane; mine[i] = c < n ? samp_keys[row * n + c] : 0; }
+  float err;
+  {  // ||bf16(q^) - q^||, q^ = q * inv_q rounded as the prepare kernel rounded it
+    const float4 v = *reinterpret_cast<const float4*>(q + row * 128 + 4 * lane);
+    const float iq = inv_q[row];
+    const uint2 w = *reinterpret_cast<const uint2*>(qn + row * 128 + 4 * lane);
+    const float2 lo = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&w.x));
+    const float2 hi = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&w.y));
+    const float a = __fmul_rn(v.x, iq) - lo.x, b = __fmul_rn(v.y, iq) - lo.y, c = __fmul_rn(v.z, iq) - hi.x, d = __fmul_rn(v.w, iq) - hi.y;
+    float es = a * a + b * b + c * c + d * d;
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) es += __shfl_xor_sync(0xffffffffu, es, o);
+    if (lane == 0) err_q[row] = sqrtf(es);
+    err = tk_err(sqrtf(es), err_t);
+  }
   int kth = 0;
   for (int r = 0; r < k; ++r) {
     int best = 0, at = 0;
@@ -419,7 +473,7 @@ __global__ void __launch_bounds__(256) topk_tau_kernel(const int* __restrict__ s
     }
     kth = wbest;
   }
-  if (lane == 0) tau[row] = kth > 0 ? fmaxf(__int_as_float(kth & ~0x1F) - (2.f * kTkErrBound + 1e-4f), 0.f) : 0.f;
+  if (lane == 0) tau[row] = kth > 0 ? fmaxf(__int_as_float(kth & ~0x1F) - (2.f * err + 1e-4f), 0.f) : 0.f;
   pdl_launch_dependents();   // (an exited thread counts as well)
 }
 
@@ -433,6 +487,7 @@ __global__ void __launch_bounds__(32 * kTkRescoreWarps) topk_rescore_kernel(cons
                                                            const float* __restrict__ table, const float* __restrict__ inv_t,
                                                            const unsigned* __restrict__ cand_grp, const unsigned* __restrict__ cand_mask,
                                                            const int* __restrict__ cand_cnt, const float* __restrict__ tau,
+                                                           const float* __restrict__ err_q, const unsigned* __restrict__ err_t,
                                                            int n_lists, long long B, long long N, int k,
                                                            long long* __restrict__ out_idx, float* __restrict__ out_score,
                                                            int* __restrict__ flag) {
@@ -540,7 +595,7 @@ __global__ void __launch_bounds__(32 * kTkRescoreWarps) topk_rescore_kernel(cons
     __syncwarp();
   }
   // nothing outside the candidate set can reach the k-th exact score: its bf16 score is <= tau
-  if (lane == 0) flag[row] = (kth > tau[row] + kTkErrBound) ? 0 : 4;
+  if (lane == 0) flag[row] = (kth > tau[row] + tk_err(err_q[row], err_t)) ? 0 : 4;   // (e_q: topk_tau_kernel)
 }
 
 // ------------------------------------------------------------------------------------------------ general path: select
@@ -717,10 +772,12 @@ __global__ void __launch_bounds__(256) topk_exact_kernel(const float* __restrict
       mys[filled * nt] = d; myi[filled * nt] = static_cast<int>(e); ++filled;
       if (filled == k) { float mn = mys[0]; for (int j = 1; j < k; ++j) mn = fminf(mn, mys[j * nt]); tau = mn; }
     } else if (d > tau) {          // replace this thread's smallest; the new smallest comes out of the same scan
-      int at = 0; float mn = mys[0], mn2 = 3.0e38f;
+      // among equal smallest scores the highest index goes (ties: lower index first); slots are not in index order
+      int at = 0, ai = myi[0]; float mn = mys[0], mn2 = 3.0e38f;
       for (int j = 1; j < k; ++j) {
         const float v = mys[j * nt];
-        if (v < mn) { mn2 = mn; mn = v; at = j; } else mn2 = fminf(mn2, v);
+        const int vi = myi[j * nt];
+        if (v < mn || (v == mn && vi > ai)) { mn2 = mn; mn = v; at = j; ai = vi; } else mn2 = fminf(mn2, v);
       }
       mys[at * nt] = d; myi[at * nt] = static_cast<int>(e);
       tau = fminf(mn2, d);
